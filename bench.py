@@ -3,7 +3,7 @@
 accept/reject), the metric of BASELINE.json.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c3|c5|ns_c4] [--scaling strong|weak]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 A "step" is one refill: `mcmc_steps` MCMC steps of every chain of the batch (one call of Sampler._mcmc_sample,
 nnest/sampler.py:229) on synthetic inputs of the named shape.  Default workload `c4` = BASELINE.json configs[3], the
@@ -26,6 +26,9 @@ GPU fixed (N independent shards, same collectives).
            over the whole gathered batch (NSBook.bulk -> nnb_ns_consume, nested.py:429-439), replicated on every rank.
 `--impl reference` times the reference's own Sampler._mcmc_sample (UNMODIFIED, installed under oracle/_ref by
 oracle/build_ref.py; the oracle port if that is absent) on the host cores, on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step handed its caller -- the gathered start points, end points and end
+loglikes of every chain, and the step's scale and counters -- to DIR/<name>.npy, so that two builds can be compared output
+for output: the inputs depend only on the arguments.
 Prints ONE JSON line.
 """
 import argparse
@@ -270,6 +273,28 @@ def cpu_baseline_quick(name, wl, budget_s=15.0):
                 else 'oracle port, per-row prior/likelihood loops as in the reference')}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, per_chain, scalars, seed=0):
+    """Writes every array to out_dir/<name>.npy (float32 arrays stay float32, all others become float64).  `per_chain`
+    arrays have one row per chain; if together they exceed DUMP_LIMIT_BYTES, the same seeded sample of rows is kept of
+    each and chain_index.npy names the rows kept."""
+    per_chain = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in per_chain.items()}
+    scalars = {k: np.atleast_1d(np.asarray(v, dtype=np.float64)) for k, v in scalars.items()}
+    n = len(next(iter(per_chain.values())))
+    row_bytes = sum(v.nbytes for v in per_chain.values()) // max(n, 1)
+    budget = DUMP_LIMIT_BYTES - sum(v.nbytes for v in scalars.values())
+    if n * row_bytes > budget:
+        keep = budget // (row_bytes + 8)
+        rows = np.sort(np.random.RandomState(seed).choice(n, keep, replace=False))
+        per_chain = {k: v[rows] for k, v in per_chain.items()}
+        per_chain['chain_index'] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in list(per_chain.items()) + list(scalars.items()):
+        np.save(os.path.join(out_dir, k + '.npy'), np.ascontiguousarray(v))
+
+
 def roofline_traffic(kernel_key, n, S):
     """dram bytes per launch from the tracked profile summary (profiles/roofline_traffic.json, written by
     profiles/ncu_summary.py from an `ncu --set full` capture), scaled to this launch's proposals."""
@@ -420,6 +445,10 @@ def run_gpu(args, name, wl):
     clk = clocks.stop() if rank == 0 else None
     proposals = n_total * S * args.steps
     value = proposals / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'first_x': ends[0].cpu().numpy(), 'last_x': ends[1].cpu().numpy(),
+                                         'last_logl': ends[2].cpu().numpy()},
+                     {'scale': last['scale'], 'naccept': naccept, 'ncall': ncall}, seed=args.seed)
 
     # ---- end-to-end arm: the repo's Python API, host arrays in, host live-point replacement out ----------------------
     from nnest_b200 import NestedSampler, MCMCSampler
@@ -600,7 +629,11 @@ def main():
     ap.add_argument('--chains', type=int, default=0, help='development: override the chains of the workload')
     ap.add_argument('--mcmc-steps', type=int, default=0, help='development: override the MCMC steps per refill')
     ap.add_argument('--fixed-scale', action='store_true', help='development: dynamic_step_size=False')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the end states of the last timed step to DIR/<name>.npy (proposals/s workloads on the GPU)')
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload == 'ns_c4' or args.impl == 'reference'):
+        ap.error('--dump-outputs is implemented for the proposals/s workloads (c2, c3, c4, c5) with --impl b200')
     if args.workload == 'ns_c4':
         import bench_ns
         return bench_ns.main(args)

@@ -38,8 +38,7 @@ def main(args):
     chains = nlive // world if args.scaling == 'strong' else nlive
     ns_iters = int(os.environ.get('NNB_NS_ITERS', 3 * nlive))
     train_iters, batch_size = 50, 8192
-    steps = max(1, min(args.steps, 5))
-    warmup = max(0, min(args.warmup, 1))
+    steps, warmup = args.steps, args.warmup
     parts = {}
 
     def timed(obj, name, key, sync=True):
