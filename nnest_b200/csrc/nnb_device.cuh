@@ -107,18 +107,35 @@ __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_
   return make_uint4(c0, c1, c2, c3);
 }
 
-// Two standard normals from two 32-bit words (Box-Muller; u1 in (0,1], angle in [-pi, pi)).
-__device__ __forceinline__ void box_muller(uint32_t ra, uint32_t rb, float& n0, float& n1) {
-  const float k2m24 = 1.0f / 16777216.0f;
-  float u1 = __fmul_rn(__fadd_rn((float)(ra >> 8), 1.0f), k2m24);
-  float u2 = __fmul_rn((float)(rb >> 8), k2m24);
-  float rad;   // sqrt(-2 ln u1): MUFU-based square root (2 ulp) instead of the ~8-instruction IEEE sequence
-  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad) : "f"(__fmul_rn(-2.0f, __logf(u1))));
-  float ang = __fmul_rn(__fsub_rn(u2, 0.5f), 6.283185307179586f);
-  float s, c;
-  __sincosf(ang, &s, &c);
-  n0 = rad * c;
-  n1 = rad * s;
+// Four standard normals from one Philox block: Box-Muller on the word pairs (r.x, r.y) -> nrm[0..1] and (r.z, r.w) ->
+// nrm[2..3] (u1 in (0,1], angle in [-pi, pi)).  The two transforms run side by side as packed FP32 pairs (FADD2 / FMUL2,
+// sm_100): each lane is rounded exactly like the scalar instruction, so the normals are the bits of two scalar transforms.
+// (ptxas may contract u2's product with the `- 0.5` into an FFMA2: that product is exact, so the bits do not change.)
+__device__ __forceinline__ void box_muller4(uint4 r, float (&nrm)[4]) {
+  const float2 k2m24 = make_float2(1.0f / 16777216.0f, 1.0f / 16777216.0f);
+  const float2 u1 = __fmul2_rn(__fadd2_rn(make_float2((float)(r.x >> 8), (float)(r.z >> 8)), make_float2(1.0f, 1.0f)), k2m24);
+  const float2 u2 = __fmul2_rn(make_float2((float)(r.y >> 8), (float)(r.w >> 8)), k2m24);
+  // -2 ln u1 = lg2(u1) * (-2 fl(ln 2)), the bits of -2.0f * __logf(u1) (= -2 * fl(lg2(u1) * fl(ln 2))): u1 >= 2^-24 is never
+  // a denormal, so the ftz lg2 returns what the denormal-guarded one inside __logf does, and -2 fl(ln 2) is exact, so one
+  // rounded product by it equals the rounded product by fl(ln 2) times -2 (scaling by a power of two commutes with rounding).
+  float2 lg;
+  asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg.x) : "f"(u1.x));
+  asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg.y) : "f"(u1.y));
+  const float2 m2ln2 = make_float2(-2.0f * 0.693147182464599609375f, -2.0f * 0.693147182464599609375f);
+  const float2 rr = __fmul2_rn(lg, m2ln2);
+  float rad0, rad1;   // sqrt(-2 ln u1): MUFU-based square root (2 ulp) instead of the ~8-instruction IEEE sequence
+  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad0) : "f"(rr.x));
+  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad1) : "f"(rr.y));
+  const float2 ang = __fmul2_rn(__fadd2_rn(u2, make_float2(-0.5f, -0.5f)), make_float2(6.283185307179586f, 6.283185307179586f));
+  float s0, c0, s1, c1;
+  __sincosf(ang.x, &s0, &c0);
+  __sincosf(ang.y, &s1, &c1);
+  const float2 n01 = __fmul2_rn(make_float2(rad0, rad0), make_float2(c0, s0));
+  const float2 n23 = __fmul2_rn(make_float2(rad1, rad1), make_float2(c1, s1));
+  nrm[0] = n01.x;
+  nrm[1] = n01.y;
+  nrm[2] = n23.x;
+  nrm[3] = n23.y;
 }
 
 __device__ __forceinline__ float uniform01(uint32_t r) { return __fmul_rn((float)(r >> 8), 1.0f / 16777216.0f); }

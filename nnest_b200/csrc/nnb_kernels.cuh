@@ -158,9 +158,7 @@ struct SmemRow {
 // normals for dims 4j..4j+3 of (chain, step)
 __device__ __forceinline__ void philox_normals4(unsigned int j, unsigned int step, unsigned int chain, unsigned int tag,
                                                 unsigned int k0, unsigned int k1, float (&nrm)[4]) {
-  uint4 r = philox4x32_10(j, step, chain, tag, k0, k1);
-  box_muller(r.x, r.y, nrm[0], nrm[1]);
-  box_muller(r.z, r.w, nrm[2], nrm[3]);
+  box_muller4(philox4x32_10(j, step, chain, tag, k0, k1), nrm);
 }
 
 struct InitParams {

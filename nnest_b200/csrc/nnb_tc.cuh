@@ -228,6 +228,19 @@ __device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) 
   hi = __float_as_uint(x) & 0xffffe000u;
   lo = __float_as_uint(x - __uint_as_float(hi));
 }
+// the same split of N values, the subtractions as packed FP32 pairs (FADD2 rounds each lane like FADD: the same bits)
+template <int N>
+__device__ __forceinline__ void split_tf32(const float* x, uint32_t* hi, uint32_t* lo) {
+#pragma unroll
+  for (int j = 0; j + 1 < N; j += 2) {
+    hi[j] = __float_as_uint(x[j]) & 0xffffe000u;
+    hi[j + 1] = __float_as_uint(x[j + 1]) & 0xffffe000u;
+    const float2 l = __fadd2_rn(make_float2(x[j], x[j + 1]), make_float2(-__uint_as_float(hi[j]), -__uint_as_float(hi[j + 1])));
+    lo[j] = __float_as_uint(l.x);
+    lo[j + 1] = __float_as_uint(l.y);
+  }
+  if (N & 1) split_tf32(x[N - 1], hi[N - 1], lo[N - 1]);
+}
 
 // host mirror of cvt.rna.tf32.f32 (round half away from zero on the magnitude), used to pre-split weights
 inline float host_rna_tf32(float x) {

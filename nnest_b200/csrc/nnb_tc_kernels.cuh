@@ -63,19 +63,30 @@ __host__ __device__ inline bool tc_supported(const FlowDesc& f) {
 //   matters for the sums the activations feed),   exp(-log_s) = 2^{l'},   log-det = ln 2 * sum l'.
 constexpr float kTcTanhScale = 2.885390081777927f;    // 2 log2(e)
 constexpr float kTcExpScale = -1.4426950408889634f;   // -log2(e)
-__device__ __forceinline__ float tc_tanh_scaled(float xs) {
-  float e;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(xs));
-  float rc;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc) : "f"(e + 1.0f));
-  return fmaf(-2.0f, rc, 1.0f);
-}
 __device__ __forceinline__ float tc_exp2(float x) {
   float e;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(x));
   return e;
 }
+__device__ __forceinline__ float tc_rcp(float x) {
+  float r;
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+  return r;
+}
+// two tanh side by side: the add and the FMA as packed FP32 pairs (each lane rounded like FADD / FFMA)
+__device__ __forceinline__ float2 tc_tanh_scaled2(float2 xs) {
+  const float2 e1 = __fadd2_rn(make_float2(tc_exp2(xs.x), tc_exp2(xs.y)), make_float2(1.0f, 1.0f));
+  return __ffma2_rn(make_float2(-2.0f, -2.0f), make_float2(tc_rcp(e1.x), tc_rcp(e1.y)), make_float2(1.0f, 1.0f));
+}
+// z' = z + scale * n of two dims, the bits of __fadd_rn(z, __fmul_rn(n, scale)) in each lane: the products as one packed
+// pair, the adds scalar.  (ptxas of CUDA 12.9 contracts a packed multiply that feeds a packed add into one FFMA2 even for
+// the .rn forms -- one rounding instead of two, other bits -- so no packed product here goes straight into a packed add.)
+__device__ __forceinline__ float2 tc_propose2(float2 z, float2 n, float scale) {
+  const float2 ns = __fmul2_rn(n, make_float2(scale, scale));
+  return make_float2(__fadd_rn(z.x, ns.x), __fadd_rn(z.y, ns.y));
+}
 
+// Philox blocks drawn side by side (c4, B200, with the packed epilogues: 2 and 8 within 0.3 % of 4)
 #ifndef NNB_TC_PHILOX_ILP
 #define NNB_TC_PHILOX_ILP 4
 #endif
@@ -168,23 +179,31 @@ __device__ __forceinline__ void tc_round_trip(TcTile& t, F0 issue0, F1 issue1) {
 template <int NPART>
 __device__ __forceinline__ void tc_hidden_epilogue(const TcTile& t, const float* __restrict__ bias) {
   if (NPART == 1) {
-    // one thread per chain: all 32 pre-activations arrive with ONE tcgen05.ld (one TMEM latency instead of four); the four
-    // chunks are then independent work for the scheduler
+    // one thread per chain: all 32 pre-activations arrive with ONE tcgen05.ld (one TMEM latency instead of four); the two
+    // nets' halves are then independent work for the scheduler, each leaving with one tcgen05.st per hi / lo half
     uint32_t r[32];
     tc::tmem_ld32(t.lane_tmem + 64, r);
     tc::wait_ld();
 #pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      uint32_t hi[8], lo[8];
-      float v[8];
+    for (int c = 0; c < 2; ++c) {
+      uint32_t hi[16], lo[16];
+      float v[16];
 #pragma unroll
-      for (int j = 0; j < 8; ++j) v[j] = __uint_as_float(r[8 * c + j]) + bias[8 * c + j];
+      for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(r[16 * c + j]) + bias[16 * c + j];
+      if (c == 0) {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) v[j] = c < 2 ? tc_tanh_scaled(v[j]) : fmaxf(v[j], 0.f);
+        for (int j = 0; j < 16; j += 2) {
+          const float2 th = tc_tanh_scaled2(make_float2(v[j], v[j + 1]));
+          v[j] = th.x;
+          v[j + 1] = th.y;
+        }
+      } else {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) tc::split_tf32(v[j], hi[j], lo[j]);
-      tc::tmem_st8(t.lane_tmem + 8 * c, hi);
-      tc::tmem_st8(t.lane_tmem + 32 + 8 * c, lo);
+        for (int j = 0; j < 16; ++j) v[j] = fmaxf(v[j], 0.f);
+      }
+      tc::split_tf32<16>(v, hi, lo);
+      tc::tmem_st16(t.lane_tmem + 16 * c, hi);
+      tc::tmem_st16(t.lane_tmem + 32 + 16 * c, lo);
     }
     return;
   }
@@ -199,15 +218,73 @@ __device__ __forceinline__ void tc_hidden_epilogue(const TcTile& t, const float*
     for (int j = 0; j < 8; ++j) v[j] = __uint_as_float(r[j]) + bias[8 * c + j];
     if (c < 2) {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) v[j] = tc_tanh_scaled(v[j]);
+      for (int j = 0; j < 8; j += 2) {
+        const float2 th = tc_tanh_scaled2(make_float2(v[j], v[j + 1]));
+        v[j] = th.x;
+        v[j + 1] = th.y;
+      }
     } else {
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = fmaxf(v[j], 0.f);
     }
-#pragma unroll
-    for (int j = 0; j < 8; ++j) tc::split_tf32(v[j], hi[j], lo[j]);
+    tc::split_tf32<8>(v, hi, lo);
     tc::tmem_st8(t.lane_tmem + 8 * c, hi);
     tc::tmem_st8(t.lane_tmem + 32 + 8 * c, lo);
+  }
+}
+
+// Output epilogue of a coupling block, columns o = ob + j (j < W) of the dims it transforms (dim o0 + 2 o).
+// yv <- the dims' current values (src 0: y; 1: nz; 2: the proposal z + scale * n, also written back to nz).  Loads first,
+// then the stores (see batched<>).
+template <int W>
+__device__ __forceinline__ void tc_out_y(float* yv, int ob, int nout, int o0, int ys, int src, const float* y,
+                                         const float* zc, float* nz, float scale) {
+#pragma unroll
+  for (int j = 0; j < W; j += 2) {
+    const int o = ob + j, i = o0 + 2 * o;
+    if (src == 2 && o + 1 < nout) {
+      const float2 zz = tc_propose2(make_float2(zc[i * ys], zc[(i + 2) * ys]), make_float2(nz[i * ys], nz[(i + 2) * ys]), scale);
+      yv[j] = zz.x;
+      yv[j + 1] = zz.y;
+    } else {
+#pragma unroll
+      for (int q = 0; q < 2; ++q)
+        if (o + q < nout) {
+          const int iq = i + 2 * q;
+          yv[j + q] = src == 2 ? __fadd_rn(zc[iq * ys], __fmul_rn(nz[iq * ys], scale)) : (src == 1 ? nz[iq * ys] : y[iq * ys]);
+        }
+    }
+  }
+  if (src == 2) {
+#pragma unroll
+    for (int j = 0; j < W; ++j)
+      if (ob + j < nout) nz[(o0 + 2 * (ob + j)) * ys] = yv[j];
+  }
+}
+// x = (y - t) * 2^{l'} of the same columns (0 past nout), ld += l' in column order (l' = -log2(e) log_s).  The bias adds
+// stay scalar (constant-bank operands); the subtract and the multiply run as packed FP32 pairs.
+template <int W>
+__device__ __forceinline__ void tc_out_x(const uint32_t* rs, const uint32_t* rt, const float* yv,
+                                         const float* __restrict__ b3s, const float* __restrict__ b3t, int ob, int nout,
+                                         float* xv, float& ld) {
+#pragma unroll
+  for (int j = 0; j < W; j += 2) {
+    const int o = ob + j;
+    xv[j] = xv[j + 1] = 0.f;
+    if (o + 1 < nout) {
+      const float ls0 = __uint_as_float(rs[j]) + b3s[o], ls1 = __uint_as_float(rs[j + 1]) + b3s[o + 1];
+      const float tt0 = __uint_as_float(rt[j]) + b3t[o], tt1 = __uint_as_float(rt[j + 1]) + b3t[o + 1];
+      const float2 x2 = __fmul2_rn(__fadd2_rn(make_float2(yv[j], yv[j + 1]), make_float2(-tt0, -tt1)),
+                                   make_float2(tc_exp2(ls0), tc_exp2(ls1)));
+      xv[j] = x2.x;
+      xv[j + 1] = x2.y;
+      ld += ls0;
+      ld += ls1;
+    } else if (o < nout) {
+      const float ls = __uint_as_float(rs[j]) + b3s[o], tt = __uint_as_float(rt[j]) + b3t[o];
+      xv[j] = (yv[j] - tt) * tc_exp2(ls);
+      ld += ls;
+    }
   }
 }
 
@@ -246,16 +323,24 @@ __device__ __forceinline__ float tc_flow_inverse(const TcFlowDesc& f, const floa
         uint32_t hi[8], lo[8];
         float v[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int a = c0 + j, i = i0 + 2 * a;
-          v[j] = a < nin ? (fused ? __fadd_rn(zc[i * ys], __fmul_rn(nz[i * ys], scale)) : y[i * ys]) : 0.f;
+        for (int j = 0; j < 8; j += 2) {
+          const int a = c0 + j, i = i0 + 2 * a;   // inputs a, a + 1 = dims i, i + 2
+          if (fused && a + 1 < nin) {
+            const float2 zz = tc_propose2(make_float2(zc[i * ys], zc[(i + 2) * ys]),
+                                          make_float2(nz[i * ys], nz[(i + 2) * ys]), scale);
+            v[j] = zz.x;
+            v[j + 1] = zz.y;
+          } else {
+            v[j] = a < nin ? (fused ? __fadd_rn(zc[i * ys], __fmul_rn(nz[i * ys], scale)) : y[i * ys]) : 0.f;
+            v[j + 1] = a + 1 < nin ? y[(i + 2) * ys] : 0.f;   // (fused: a + 1 >= nin here)
+          }
         }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {   // (stores after all loads of the chunk: see batched<>)
           const int a = c0 + j, i = i0 + 2 * a;
           if (fused && a < nin) nz[i * ys] = v[j];
-          tc::split_tf32(v[j], hi[j], lo[j]);
         }
+        tc::split_tf32<8>(v, hi, lo);
         tc::tmem_st8(t.lane_tmem + c0, hi);
         tc::tmem_st8(t.lane_tmem + 32 + c0, lo);
       }
@@ -303,85 +388,55 @@ __device__ __forceinline__ float tc_flow_inverse(const TcFlowDesc& f, const floa
     // x = (z - t) * exp(-log_s), ld -= log_s on the dims with mask == 0   (networks.py:300-309).  The values a dim keeps
     // (its last update: blocks 1 and 0) are tested against the prior box right here (priors.py:39-43).
     const bool chk = box_check && k <= 1;
+    // where y of a transformed dim comes from: the proposal z + scale * n formed here (first block of a fused flow), the
+    // first block's output left in nz (second block of a fused flow), or y
+    const int ysrc = fused && k == nB - 1 ? 2 : (fused && k == nB - 2 ? 1 : 0);
     if (NPART == 1 && N3 == 16) {
-      // one thread per chain, at most 16 transformed dims: both output rows arrive before a single wait
-      uint32_t rs[16], rt[16];
+      // one thread per chain, at most 16 transformed dims: both output rows arrive before a single wait, and the A operand
+      // of the next block leaves with one tcgen05.st per half (columns past nout: zeros, never read by layer 1)
+      uint32_t rs[16], rt[16], hi[16], lo[16];
       tc::tmem_ld16(t.lane_tmem + 64, rs);
       tc::tmem_ld16(t.lane_tmem + t_col, rt);
       float yv[16];   // the dims this block transforms, read before any of them is written back (see batched<>)
-#pragma unroll
-      for (int o = 0; o < 16; ++o) {
-        const int i = o0 + 2 * o;
-        if (o < nout)
-          yv[o] = (fused && k == nB - 1) ? __fadd_rn(zc[i * ys], __fmul_rn(nz[i * ys], scale))
-                                         : ((fused && k == nB - 2) ? nz[i * ys] : y[i * ys]);
-      }
-      if (fused && k == nB - 1) {
-#pragma unroll
-        for (int o = 0; o < 16; ++o)
-          if (o < nout) nz[(o0 + 2 * o) * ys] = yv[o];
-      }
+      tc_out_y<16>(yv, 0, nout, o0, ys, ysrc, y, zc, nz, scale);
       tc::wait_ld();
 #pragma unroll
       for (int c0 = 0; c0 < 16; c0 += 8) {
-        if (c0 < nout) {
-          uint32_t hi[8], lo[8];
+        float xv[8];
+        tc_out_x<8>(rs + c0, rt + c0, yv + c0, b3s, b3t, c0, nout, xv, ld);
 #pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const int o = c0 + j;
-            float xv = 0.f;
-            if (o < nout) {
-              const float ls = __uint_as_float(rs[o]) + b3s[o];
-              const float tt = __uint_as_float(rt[o]) + b3t[o];
-              float* yp = y + (o0 + 2 * o) * ys;
-              xv = (yv[o] - tt) * tc_exp2(ls);   // ls = -log2(e) log_s
-              *yp = xv;
-              ld += ls;
-              if (chk) bad |= (xv < lof[o0 + 2 * o]) | (xv > hif[o0 + 2 * o]);
-            }
-            tc::split_tf32(xv, hi[j], lo[j]);
-          }
-          if (k > 0) {   // A operand of block k-1's first layer
-            tc::tmem_st8(t.lane_tmem + c0, hi);
-            tc::tmem_st8(t.lane_tmem + 32 + c0, lo);
+        for (int j = 0; j < 8; ++j) {
+          const int o = c0 + j;
+          if (o < nout) {
+            y[(o0 + 2 * o) * ys] = xv[j];
+            if (chk) bad |= (xv[j] < lof[o0 + 2 * o]) | (xv[j] > hif[o0 + 2 * o]);
           }
         }
+        tc::split_tf32<8>(xv, hi + c0, lo + c0);
+      }
+      if (k > 0) {   // A operand of block k-1's first layer
+        tc::tmem_st16(t.lane_tmem, hi);
+        tc::tmem_st16(t.lane_tmem + 32, lo);
       }
     } else {
     for (int c0 = (NPART == 1 ? 0 : 8 * t.part); c0 < nout; c0 += 8 * NPART) {
       uint32_t rs[8], rt[8], hi[8], lo[8];
       tc::tmem_ld8(t.lane_tmem + 64 + c0, rs);
       tc::tmem_ld8(t.lane_tmem + t_col + c0, rt);
-      float yv[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const int i = o0 + 2 * (c0 + j);
-        if (c0 + j < nout)
-          yv[j] = (fused && k == nB - 1) ? __fadd_rn(zc[i * ys], __fmul_rn(nz[i * ys], scale))
-                                         : ((fused && k == nB - 2) ? nz[i * ys] : y[i * ys]);
-      }
-      if (fused && k == nB - 1) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-          if (c0 + j < nout) nz[(o0 + 2 * (c0 + j)) * ys] = yv[j];
-      }
+      float yv[8], xv[8];
+      tc_out_y<8>(yv, c0, nout, o0, ys, ysrc, y, zc, nz, scale);
       tc::wait_ld();
+      tc_out_x<8>(rs, rt, yv, b3s, b3t, c0, nout, xv, ld);
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         const int o = c0 + j;
-        float xv = 0.f;
         if (o < nout) {
-          const float ls = __uint_as_float(rs[j]) + b3s[o];
-          const float tt = __uint_as_float(rt[j]) + b3t[o];
-          float* yp = y + (o0 + 2 * o) * ys;
-          xv = (yv[j] - tt) * tc_exp2(ls);   // ls = -log2(e) log_s
-          *yp = xv;
-          ld += ls;
-          if (chk) bad |= (xv < lof[o0 + 2 * o]) | (xv > hif[o0 + 2 * o]);
+          y[(o0 + 2 * o) * ys] = xv[j];
+          if (chk) bad |= (xv[j] < lof[o0 + 2 * o]) | (xv[j] > hif[o0 + 2 * o]);
         }
-        tc::split_tf32(xv, hi[j], lo[j]);
       }
       if (k > 0) {   // A operand of block k-1's first layer
+        tc::split_tf32<8>(xv, hi, lo);
         tc::tmem_st8(t.lane_tmem + c0, hi);
         tc::tmem_st8(t.lane_tmem + 32 + c0, lo);
       }
@@ -649,7 +704,8 @@ mcmc_tc_kernel(TcFlowDesc f, const float* __restrict__ wglob, TargetDesc td, con
       NNB_TSTAMP(0);
       // The tiles of an SM leave the grid barrier together and would then all run their epilogues at the same moments and
       // all wait for their MMAs at the same moments; odd tiles therefore start the step about half a round trip late
-      // (p.tc_delay, NNB_TC_DELAYS; measured on the B200 at c4: 2.23 ms -> 2.14 ms per refill at 700 cycles)
+      // (p.tc_delay, NNB_TC_DELAYS; measured on the B200 at c4: 2.23 ms -> 2.14 ms per refill at 700 cycles; re-swept with the
+      // packed epilogues (1.82 ms): 500 / 900 cycles within 0.3 % of 700, no delay +1.2 %)
       if (p.tc_delay[tile & 3] > 0) {
         const long long t0 = clock64();
         while (clock64() - t0 < (long long)p.tc_delay[tile & 3]) {}
@@ -735,15 +791,27 @@ mcmc_tc_kernel(TcFlowDesc f, const float* __restrict__ wglob, TargetDesc td, con
             if (DD > 0 && td.like_id == NNB_LIKE_ROSENBROCK && !td.compute_f64 && td.has_transform) {
               // the config-4 target inline (same arithmetic as loglike_T<float>: likelihoods.py:50-51 after the float32
               // affine transform), transform coefficients as constant-bank operands
-              constexpr int D1 = DD > 0 ? DD : 1;
-              float acc = 0.f, prev = __fadd_rn(__fmul_rn(y[0], cst_t[0]), cst_t[D1]);
-              batched<kCh>(D1 - 1, [&](int i) { return __fadd_rn(__fmul_rn(y[(i + 1) * 128], cst_t[i + 1]), cst_t[D1 + i + 1]); },
-                           [&](int, float cur) {
-                             const float t1 = __fsub_rn(cur, __fmul_rn(prev, prev));
-                             const float t2 = __fsub_rn(1.f, prev);
-                             acc = __fadd_rn(acc, __fadd_rn(__fmul_rn(100.f, __fmul_rn(t1, t1)), __fmul_rn(t2, t2)));
-                             prev = cur;
-                           });
+              // The terms i = 1 .. N run as packed FP32 pairs (i, i + h), h = ceil(N / 2): with V_m = (x_m, x_{m+h}) a pair's
+              // current and previous values are V_i and V_{i-1}.  acc still adds the terms in the order i = 1 .. N: the first
+              // lanes as they come, then the second lanes (terms h+1 .. N).
+              constexpr int D1 = DD > 0 ? DD : 1, N = D1 - 1, h = (N + 1) / 2;
+              auto xt = [&](int i) { return i < D1 ? __fadd_rn(__fmul_rn(y[i * 128], cst_t[i]), cst_t[D1 + i]) : 0.f; };
+              float acc = 0.f, late[h > 0 ? h : 1];
+              float2 prev = make_float2(xt(0), xt(h));
+#pragma unroll
+              for (int i = 1; i <= h; ++i) {
+                const float2 cur = make_float2(xt(i), xt(i + h));
+                // (the adds that take a product are scalar: see tc_propose2)
+                const float2 sq = __fmul2_rn(prev, prev);
+                const float2 t1 = make_float2(__fsub_rn(cur.x, sq.x), __fsub_rn(cur.y, sq.y));
+                const float2 t2 = __fadd2_rn(make_float2(1.f, 1.f), make_float2(-prev.x, -prev.y));
+                const float2 a = __fmul2_rn(make_float2(100.f, 100.f), __fmul2_rn(t1, t1)), b = __fmul2_rn(t2, t2);
+                acc = __fadd_rn(acc, __fadd_rn(a.x, b.x));
+                late[i - 1] = __fadd_rn(a.y, b.y);   // term i + h (i + h > N: the padding lane, unused)
+                prev = cur;
+              }
+#pragma unroll
+              for (int i = h + 1; i <= N; ++i) acc = __fadd_rn(acc, late[i - h - 1]);
               const double out = -(double)acc;
               lp = isfinite(out) ? out : (double)-INFINITY;   // float32-typed result: sampler.py:128 leaves -inf
             } else {
