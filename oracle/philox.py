@@ -6,7 +6,8 @@ The reference draws from torch's global CPU generator (sampler.py:310,334,377,41
 be reproduced on a GPU; north_star replaces it by a counter-based Philox stream keyed per chain.
 This module is the executable specification of that stream (documented in DESIGN.md):
   key     = (seed & 0xffffffff, seed >> 32)
-  counter = (j, step, chain, tag)   tag 0: proposal normals, 1: accept uniform, 2: start latents
+  counter = (j, step, chain, tag)   tag 0: proposal normals, 1: accept uniform, 2: start latents,
+                                    3: jitter of the flow-fitting data (step = epoch, chain = position in the epoch)
   normals for dims 4j..4j+3 come from the four outputs of counter word j (two Box-Muller pairs)
 Pinned by the Random123 known-answer vectors in tests/test_oracle_philox.py.
 """
@@ -17,7 +18,7 @@ M1 = np.uint64(0xCD9E8D57)
 W0 = 0x9E3779B9
 W1 = 0xBB67AE85
 MASK = np.uint64(0xFFFFFFFF)
-TAG_NORMAL, TAG_UNIFORM, TAG_INIT = 0, 1, 2
+TAG_NORMAL, TAG_UNIFORM, TAG_INIT, TAG_TRAIN = 0, 1, 2, 3
 TWO_M24 = np.float32(1.0 / 16777216.0)
 
 

@@ -82,19 +82,21 @@ def _mlp_backward(layers, glayers, kind, acts, dout):
     return dh
 
 
-def nll_and_grad(flat, x, d, H, L, B, want_grad=True):
-    """-log p(x) per sample (n,), and the gradient of mean(-log p) with respect to the flat parameters."""
-    flat = np.asarray(flat, dtype=np.float64)
-    x = np.asarray(x, dtype=np.float64)
+def nll_and_grad(flat, x, d, H, L, B, want_grad=True, dtype=np.float64):
+    """-log p(x) per sample (n,), and the gradient of mean(-log p) with respect to the flat parameters.
+    dtype=np.float32 runs the same arithmetic in float32: its distance from the float64 result measures how well a float32
+    implementation can do on the given inputs."""
+    flat = np.asarray(flat, dtype=dtype)
+    x = np.asarray(x, dtype=dtype)
     n = x.shape[0]
     nP = net_floats(d, H, L)
     nets = [(_split_net(flat[(2 * k) * nP:(2 * k + 1) * nP], d, H, L),
              _split_net(flat[(2 * k + 1) * nP:(2 * k + 2) * nP], d, H, L)) for k in range(B)]
     saved = []
     y = x
-    ld = np.zeros(n)
+    ld = np.zeros(n, dtype=dtype)
     for k in range(B):
-        mask = ((np.arange(d) + k) % 2).astype(np.float64)
+        mask = ((np.arange(d) + k) % 2).astype(dtype)
         xm = y * mask
         s, acts_s = _mlp_forward(nets[k][0], 0, xm)
         t, acts_t = _mlp_forward(nets[k][1], 1, xm)
@@ -104,7 +106,7 @@ def nll_and_grad(flat, x, d, H, L, B, want_grad=True):
         saved.append((y, mask, s, acts_s, acts_t))
         ld += s.sum(1)
         y = z
-    nll = 0.5 * (y * y).sum(1) + 0.5 * d * np.log(2 * np.pi) - ld
+    nll = 0.5 * (y * y).sum(1) + dtype(0.5 * d * np.log(2 * np.pi)) - ld
     if not want_grad:
         return nll, None
     grad = np.zeros_like(flat)
@@ -119,6 +121,28 @@ def nll_and_grad(flat, x, d, H, L, B, want_grad=True):
             _mlp_backward(nets[k][1], gnets[k][1], 1, acts_t, dt)
         gy = gy * np.exp(s) + dxm * mask
     return nll, grad
+
+
+def relu_margin(flat, x, d, H, L, B):
+    """Per sample (n,), the smallest |pre-activation| of any ReLU unit of the translate nets.  The gradient jumps where
+    one crosses 0, so where the margin is within rounding error a float32 implementation and this oracle may differ by
+    the size of the jump."""
+    flat = np.asarray(flat, dtype=np.float64)
+    y = np.asarray(x, dtype=np.float64)
+    nP = net_floats(d, H, L)
+    margin = np.full(y.shape[0], np.inf)
+    for k in range(B):
+        mask = ((np.arange(d) + k) % 2).astype(np.float64)
+        s, _ = _mlp_forward(_split_net(flat[(2 * k) * nP:(2 * k + 1) * nP], d, H, L), 0, y * mask)
+        layers = _split_net(flat[(2 * k + 1) * nP:(2 * k + 2) * nP], d, H, L)
+        h = y * mask
+        for (W, b) in layers[:-1]:
+            pre = h @ W.T + b
+            margin = np.minimum(margin, np.abs(pre).min(1))
+            h = np.maximum(pre, 0.0)
+        W, b = layers[-1]
+        y = y * np.exp(s * (1 - mask)) + (h @ W.T + b) * (1 - mask)
+    return margin
 
 
 class Adam(object):

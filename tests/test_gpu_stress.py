@@ -42,29 +42,32 @@ def test_mcmc_refill_is_bit_reproducible():
 
 
 def test_many_cta_fitting_is_bit_reproducible():
-    """32 CTAs per mini-batch: partial gradients and losses are reduced in a fixed CTA order (no floating-point atomics),
-    so identical inputs give identical bits -- weights, training loss, validation loss."""
+    """Several CTAs per mini-batch: partial gradients and losses are reduced in a fixed CTA order (no floating-point
+    atomics), so identical inputs give identical bits -- weights, Adam moments, training loss, validation loss.  Batch 4096
+    runs on 32 CTAs; batch 320 x sm_count on every SM, each CTA walking two or three 128-sample slices."""
     import bench
     from nnest_b200.engine import Engine
     eng = Engine(0)
     d = 30
+    sm = torch.cuda.get_device_properties(0).multi_processor_count
     rng = np.random.RandomState(0)
-    x = torch.from_numpy(rng.uniform(-1, 1, size=(20000, d)).astype(np.float32)).cuda()
     w0 = torch.from_numpy(bench.flat_weights(bench.make_weights(d, 0))).cuda()
-    ref = None
-    for _ in range(10):
-        w, m, v = w0.clone(), torch.zeros_like(w0), torch.zeros_like(w0)
-        steps = 0
-        for ep in range(2):
-            tl, vs, grid = eng.train_epoch((d, 16, 1, 3), w, m, v, steps, x, x[:1000].contiguous(), 4096, jitter=0.01,
-                                           lr=1e-3, weight_decay=1e-6, seed=3, epoch=ep)
-            steps += 5
-        assert grid == 32
-        if ref is None:
-            ref = (w.clone(), tl, vs)
-        else:
-            assert torch.equal(w, ref[0])
-            assert tl == ref[1] and vs == ref[2]
+    for batch, n in ((4096, 20000), (320 * sm, 640 * sm + 777)):
+        x = torch.from_numpy(rng.uniform(-1, 1, size=(n, d)).astype(np.float32)).cuda()
+        ref = None
+        for _ in range(10):
+            w, m, v = w0.clone(), torch.zeros_like(w0), torch.zeros_like(w0)
+            steps = 0
+            for ep in range(2):
+                tl, vs, grid = eng.train_epoch((d, 16, 1, 3), w, m, v, steps, x, x[:1000].contiguous(), batch,
+                                               jitter=0.01, lr=1e-3, weight_decay=1e-6, seed=3, epoch=ep)
+                steps += (n + batch - 1) // batch
+            assert grid == min(batch // 128, sm)
+            if ref is None:
+                ref = (w.clone(), m.clone(), v.clone(), tl, vs)
+            else:
+                assert torch.equal(w, ref[0]) and torch.equal(m, ref[1]) and torch.equal(v, ref[2])
+                assert tl == ref[3] and vs == ref[4]
 
 
 def test_mean_nn_distance_is_bit_reproducible():
