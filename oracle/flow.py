@@ -1,4 +1,5 @@
-"""CPU oracle: RealNVP / affine-coupling flow of the reference, restated in numpy float32.
+"""CPU oracle: RealNVP / affine-coupling flow of the reference, restated in numpy float32 (and, with dtype=np.float64,
+in float64 on the same float32 weights: a reference whose own rounding is negligible next to a float32 kernel's).
 
 TEST INFRASTRUCTURE ONLY.  Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline /
 --impl reference leg may import this module; the product package (nnest_b200) never does.
@@ -66,9 +67,12 @@ class NVPWeights(object):
         return cls(d, hidden, nl, num_blocks, blocks, translate_only)
 
     @classmethod
-    def random(cls, d, hidden=16, num_layers=1, num_blocks=3, seed=0, gain=1.0, translate_only=False):
+    def random(cls, d, hidden=16, num_layers=1, num_blocks=3, seed=0, gain=1.0, scale=''):
         """nn.Linear-style default init U(-1/sqrt(fan_in), 1/sqrt(fan_in)) from a numpy generator
-        (used where torch is not wanted; distribution only, not torch's stream)."""
+        (used where torch is not wanted; distribution only, not torch's stream).  scale: the reference's `scale` kwarg;
+        'constant' draws each block's ScaleLayer parameter from U(-0.5, 0.5), rounded to float32."""
+        assert scale in ('', 'translate', 'constant')
+        translate_only = scale != ''
         rng = np.random.default_rng(seed)
 
         def lin(o, i):
@@ -83,6 +87,8 @@ class NVPWeights(object):
                     continue
                 layers = [lin(hidden, d)] + [lin(hidden, hidden) for _ in range(num_layers)] + [lin(d, hidden)]
                 blk[net] = layers
+            if scale == 'constant':
+                blk['const_scale'] = float(F32(rng.uniform(-0.5, 0.5)))
             blocks.append(blk)
         return cls(d, hidden, num_layers, num_blocks, blocks, translate_only)
 
@@ -103,66 +109,66 @@ class NVPWeights(object):
         return np.concatenate(out)
 
 
-def _mlp(layers, act, v):
+def _mlp(layers, act, v, dtype=F32):
     # networks.py:273-282 : Linear, act, [Linear, act] x L, Linear  (no activation after the last)
     h = v
     n = len(layers)
     for j, (W, b) in enumerate(layers):
-        h = (h @ W.T + b).astype(F32)
+        h = (h @ np.asarray(W, dtype=dtype).T + np.asarray(b, dtype=dtype)).astype(dtype)
         if j < n - 1:
-            h = np.tanh(h) if act == 'tanh' else np.maximum(h, F32(0))
-    return h.astype(F32)
+            h = np.tanh(h) if act == 'tanh' else np.maximum(h, dtype(0))
+    return h.astype(dtype)
 
 
-def coupling_forward(w, k, x):
+def coupling_forward(w, k, x, dtype=F32):
     """networks.py:289-298"""
     blk = w.blocks[k]
-    mask = w.mask(k)
+    mask = w.mask(k).astype(dtype)
     masked = x * mask
-    t = _mlp(blk['translate'], 'relu', masked) * (F32(1) - mask)
+    t = _mlp(blk['translate'], 'relu', masked, dtype) * (dtype(1) - mask)
     if blk['scale'] is None:
-        return (x + t).astype(F32), np.zeros(x.shape[0], dtype=F32)
-    log_s = _mlp(blk['scale'], 'tanh', masked) * (F32(1) - mask)
+        return (x + t).astype(dtype), np.zeros(x.shape[0], dtype=dtype)
+    log_s = _mlp(blk['scale'], 'tanh', masked, dtype) * (dtype(1) - mask)
     s = np.exp(log_s)
-    return (x * s + t).astype(F32), log_s.sum(-1, dtype=F32)
+    return (x * s + t).astype(dtype), log_s.sum(-1, dtype=dtype)
 
 
-def coupling_inverse(w, k, z):
+def coupling_inverse(w, k, z, dtype=F32):
     """networks.py:300-309"""
     blk = w.blocks[k]
-    mask = w.mask(k)
+    mask = w.mask(k).astype(dtype)
     masked = z * mask
-    t = _mlp(blk['translate'], 'relu', masked) * (F32(1) - mask)
+    t = _mlp(blk['translate'], 'relu', masked, dtype) * (dtype(1) - mask)
     if blk['scale'] is None:
-        return (z - t).astype(F32), np.zeros(z.shape[0], dtype=F32)
-    log_s = _mlp(blk['scale'], 'tanh', masked) * (F32(1) - mask)
+        return (z - t).astype(dtype), np.zeros(z.shape[0], dtype=dtype)
+    log_s = _mlp(blk['scale'], 'tanh', masked, dtype) * (dtype(1) - mask)
     s = np.exp(-log_s)
-    return ((z - t) * s).astype(F32), (-log_s).sum(-1, dtype=F32)
+    return ((z - t) * s).astype(dtype), (-log_s).sum(-1, dtype=dtype)
 
 
-def flow_forward(w, x):
+def flow_forward(w, x, dtype=F32):
     """x (N,d) -> z (N,d), log_det (N,)   [networks.py:24-32, blocks in natural order]"""
-    x = np.ascontiguousarray(x, dtype=F32)
-    ld = np.zeros(x.shape[0], dtype=F32)
+    x = np.ascontiguousarray(x, dtype=dtype)
+    ld = np.zeros(x.shape[0], dtype=dtype)
     for k in range(w.num_blocks):
-        x, l = coupling_forward(w, k, x)
-        ld = (ld + l).astype(F32)
+        x, l = coupling_forward(w, k, x, dtype)
+        ld = (ld + l).astype(dtype)
         cs = w.blocks[k]['const_scale']
         if cs is not None:  # ScaleLayer.forward networks.py:319-321 (log-det is the scalar itself)
-            x = (x * np.exp(F32(cs))).astype(F32)
-            ld = (ld + F32(cs)).astype(F32)
+            x = (x * np.exp(dtype(F32(cs)))).astype(dtype)
+            ld = (ld + dtype(F32(cs))).astype(dtype)
     return x, ld
 
 
-def flow_inverse(w, z):
+def flow_inverse(w, z, dtype=F32):
     """z (N,d) -> x (N,d), log_det (N,)   [networks.py:34-42, blocks reversed]"""
-    z = np.ascontiguousarray(z, dtype=F32)
-    ld = np.zeros(z.shape[0], dtype=F32)
+    z = np.ascontiguousarray(z, dtype=dtype)
+    ld = np.zeros(z.shape[0], dtype=dtype)
     for k in range(w.num_blocks - 1, -1, -1):
         cs = w.blocks[k]['const_scale']
         if cs is not None:  # ScaleLayer.inverse networks.py:323-325 (it follows block k in the list)
-            z = (z * np.exp(-F32(cs))).astype(F32)
-            ld = (ld - F32(cs)).astype(F32)
-        z, l = coupling_inverse(w, k, z)
-        ld = (ld + l).astype(F32)
+            z = (z * np.exp(-dtype(F32(cs)))).astype(dtype)
+            ld = (ld - dtype(F32(cs))).astype(dtype)
+        z, l = coupling_inverse(w, k, z, dtype)
+        ld = (ld + l).astype(dtype)
     return z, ld

@@ -320,7 +320,7 @@ def test_mcmc_generic_tensor_core_path_matches_oracle(engine, d, layers, blocks,
     old = os.environ.get('NNB_TC_NPART')
     os.environ['NNB_TC_NPART'] = npart           # read by the library at every launch
     try:
-        _generic_case(engine, L.NNB_IMPL_TCGEN05, w, d, layers, blocks, steps, n)
+        _generic_case(engine, L.NNB_IMPL_TCGEN05, w, steps, n)
     finally:
         if old is None:
             del os.environ['NNB_TC_NPART']
@@ -335,30 +335,47 @@ def test_mcmc_generic_16_lane_path_matches_oracle(engine, d, layers, blocks):
     never transformed), more than 16 outputs per block (two per lane), more than 64 dims (two Philox blocks per lane)."""
     from nnest_b200 import _lib as L
     w = oflow.NVPWeights.random(d, hidden=16, num_layers=layers, num_blocks=blocks, seed=d, gain=1.3)
-    _generic_case(engine, L.NNB_IMPL_WARP, w, d, layers, blocks, 6, 700)
+    _generic_case(engine, L.NNB_IMPL_WARP, w, 6, 700)
 
 
-def _generic_case(engine, impl, w, d, layers, blocks, steps, n):
-    from nnest_b200 import _lib as L
-    engine.set_flow(w.flat(), d, 16, layers, blocks, 0)
-    engine.set_target(d, 0, [], t_scale=5.0, t_shift=0.0, prior_kind=1, prior_lo=-1.0, prior_hi=1.0)
+def _generic_case(engine, impl, w, steps, n, flags=0, target='rosenbrock', dynamic=True):
+    """`steps` free-running steps of `n` chains of the flow `w` (any hidden_dim / scale mode; `flags` = its nnb_set_flow
+    flags) on `impl`: Philox noise dumped by the kernel, replayed through the oracle.  target 'rosenbrock': the hard
+    constraint at the 25th percentile of the start points, with the dynamic or a fixed step size; 'gaussian': Metropolis-
+    Hastings on a float64 correlated Gaussian in transformed coordinates.  Returns (end state, mcmc_run result)."""
+    d = w.d
+    engine.set_flow(w.flat(), d, w.hidden, w.num_layers, w.num_blocks, flags)
     rng = np.random.RandomState(d)
     u0 = rng.uniform(-0.6, 0.6, size=(n, d))
-    like = olike.Rosenbrock(d)
-    logl0 = like.batch(5 * u0)
-    loglstar = float(np.percentile(logl0, 25))
+    if target == 'rosenbrock':
+        like = olike.Rosenbrock(d)
+        engine.set_target(d, 0, [], t_scale=5.0, t_shift=0.0, prior_kind=1, prior_lo=-1.0, prior_hi=1.0)
+        tgt = omcmc.Target(like, transform=lambda x: 5 * x, prior=olike.UniformPrior(d, -1, 1), transform_prior=False)
+        logl0 = like.batch(5 * u0)
+        # a fixed step stays at its start value: a third of the dynamic run's start keeps chains moving
+        mode, loglstar, step_size = 0, float(np.percentile(logl0, 25)), (1.0 if dynamic else 0.3) / d ** 0.5
+    else:
+        assert target == 'gaussian'
+        like = olike.Gaussian(d, 0.5)
+        engine.set_target(d, like.like_id, like.params(), t_scale=2.0, t_shift=0.5, compute_f64=True, prior_kind=2,
+                          prior_lo=-10.0, prior_hi=10.0)
+        tgt = omcmc.Target(like, transform=lambda x: x * 2.0 + 0.5, prior=olike.UniformPrior(d, -10, 10),
+                           transform_prior=True)
+        logl0 = tgt.loglike(u0)
+        mode, loglstar, step_size = 1, None, 0.5 / d ** 0.5
     st, _, _ = engine.mcmc_init(n, init_u=dev(np.ascontiguousarray(u0.astype(np.float32).T)), init_logl=dev(logl0),
                                 seed=11)
-    out = engine.mcmc_run(st, steps, mode=0, loglstar=loglstar, step_size=1 / d ** 0.5, dynamic_step_size=True,
+    out = engine.mcmc_run(st, steps, mode=mode, loglstar=loglstar, step_size=step_size, dynamic_step_size=dynamic,
                           seed=11, trace=True, dump_noise=True, impl=impl)
-    assert out['impl'] == impl
-    target = omcmc.Target(like, transform=lambda x: 5 * x, prior=olike.UniformPrior(d, -1, 1), transform_prior=False)
-    ref = omcmc.mcmc_sample(w, target, steps, omcmc.ReplayNoise(out['normals'].cpu().numpy(),
-                                                                 out['uniforms'].cpu().numpy()),
-                            step_size=1 / d ** 0.5, dynamic_step_size=True, init_samples=u0, init_loglikes=logl0,
+    if impl != 0:
+        assert out['impl'] == impl
+    ref = omcmc.mcmc_sample(w, tgt, steps, omcmc.ReplayNoise(out['normals'].cpu().numpy(),
+                                                              out['uniforms'].cpu().numpy()),
+                            step_size=step_size, dynamic_step_size=dynamic, init_samples=u0, init_loglikes=logl0,
                             loglstar=loglstar)
     latent = out['trace_z'].permute(2, 0, 1).cpu().numpy()
     samples = out['trace_x'].permute(2, 0, 1).cpu().numpy()
+    loglikes = out['trace_logl'].permute(1, 0).cpu().numpy()
     moved_ref = np.any(ref[1][:, 1:] != ref[1][:, :-1], axis=2)
     moved = np.any(latent[:, 1:] != latent[:, :-1], axis=2)
     same = np.all(moved == moved_ref, axis=1)
@@ -366,7 +383,13 @@ def _generic_case(engine, impl, w, d, layers, blocks, steps, n):
     assert moved.sum() > 0.1 * moved.size           # the test moves chains
     assert rel_err(latent[same], ref[1][same]) < TOL
     assert rel_err(samples[same], ref[0][same]) < TOL
+    assert rel_err(loglikes[same], ref[3][same]) < TOL
+    if (~same).sum() == 0:
+        assert out['ncall'] == ref[5]
+        assert abs(out['scale'] - ref[4]) <= 1e-12 * ref[4]
     assert torch.equal(st.z, out['trace_z'][-1]) and torch.equal(st.x, out['trace_x'][-1])
+    assert torch.equal(st.logl, out['trace_logl'][-1])
+    return st, out
 
 
 @pytest.mark.parametrize('impl', IMPLS)

@@ -14,18 +14,21 @@ FLOW_FILES = ['flow_d2.npz', 'flow_d3.npz', 'flow_d4.npz', 'flow_d5.npz', 'flow_
 TOL = 1e-5   # north_star: flow forward/inverse and log-det within 1e-5 relative
 
 
-@pytest.mark.parametrize('name', FLOW_FILES)
-def test_flow_matches_reference(name):
+# the float32 oracle keeps its original ids; the float64 oracle (the reference of the GPU flow sweep) is one more dtype
+@pytest.mark.parametrize('name,dtype', [pytest.param(n, np.float32, id=n) for n in FLOW_FILES] +
+                         [pytest.param(n, np.float64, id=n + '-float64') for n in FLOW_FILES])
+def test_flow_matches_reference(name, dtype):
     g = load(name)
     w = weights_of(g)
-    z, ld = oflow.flow_forward(w, g['x'])
+    z, ld = oflow.flow_forward(w, g['x'], dtype=dtype)
+    assert z.dtype == dtype and ld.dtype == dtype
     assert rel_err(z, g['fwd_z']) < TOL
     assert np.allclose(ld, g['fwd_ld'], rtol=TOL, atol=1e-6)
-    x, ldx = oflow.flow_inverse(w, g['zin'])
+    x, ldx = oflow.flow_inverse(w, g['zin'], dtype=dtype)
     assert rel_err(x, g['inv_x']) < TOL
     assert np.allclose(ldx, g['inv_ld'], rtol=TOL, atol=1e-6)
     # the properties tests/test_flows.py:56-72 checks on the reference
-    xr, ldr = oflow.flow_inverse(w, z)
+    xr, ldr = oflow.flow_inverse(w, z, dtype=dtype)
     assert np.abs(xr - g['x']).max() <= 2e-5
     assert np.abs(ldr + ld).max() <= 1e-5
 
