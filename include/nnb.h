@@ -22,14 +22,16 @@
 #ifndef NNB_H_
 #define NNB_H_
 
+#ifndef __CUDACC_RTC__
 #include <stddef.h>
 #include <stdint.h>
+#endif
 
 #ifdef __cplusplus
 extern "C" {
 #endif
 
-#define NNB_ABI_VERSION 13
+#define NNB_ABI_VERSION 14
 #define NNB_MAX_DIM 128      /* x_dim */
 #define NNB_MAX_BLOCKS 16    /* num_blocks */
 #define NNB_MAX_LIKE_PARAMS 160
@@ -53,7 +55,8 @@ enum {
   NNB_LIKE_GAUSSIAN = 2,       /* :77-86   params: corr */
   NNB_LIKE_EGGBOX = 3,         /* :97-106  params: none (product over all dims; reference has d == 2) */
   NNB_LIKE_GAUSSIAN_MIX = 4,   /* :165-189 params: sep, sigma, ncomp, w[ncomp] */
-  NNB_LIKE_GAUSSIAN_SHELL = 5  /* :113-128 params: sigma, rshell, center[d] */
+  NNB_LIKE_GAUSSIAN_SHELL = 5, /* :113-128 params: sigma, rshell, center[d] */
+  NNB_LIKE_USER = 6            /* the handle's user likelihood (nnb_set_user_likelihood)   params: any, up to the maximum */
 };
 
 enum { NNB_PRIOR_NONE = 0, NNB_PRIOR_BOX_U = 1, NNB_PRIOR_BOX_V = 2 };
@@ -145,6 +148,30 @@ typedef struct {
 } nnb_target;
 
 int nnb_set_target(nnb_handle* h, int d, const nnb_target* t);
+
+/*
+ * A likelihood written by the user in CUDA C++ (no counterpart in the reference, whose likelihoods are Python callables
+ * that cannot run inside the kernels).  `source` defines
+ *     template <typename X> __device__ double nnb_user_loglike(const X& x, int d, const double* params);
+ * x(i) is coordinate i after the target's transform, in the arithmetic type the built-in likelihoods see at the same place
+ * (float when compute_f64 == 0 and the input is float32, double otherwise); params are the target's like_params (up to
+ * NNB_MAX_LIKE_PARAMS).  Larger constants go into the source as __constant__ arrays.  A non-finite result becomes -inf
+ * when x(i) is float and -1e100 otherwise, as for the built-in likelihoods.
+ * nnb_set_user_likelihood installs the source on the handle; nnb_set_target with like_id NNB_LIKE_USER then selects it
+ * (NNB_ERR_STATE before a source is installed).  NVRTC compiles the library's own kernel templates around the source:
+ * the likelihood kernel during this call (NNB_ERR_ARG with NVRTC's log in nnb_last_error when the source does not
+ * compile), every other kernel variant the first time a call runs it.  Compiled variants are kept per handle and on
+ * disk under $NNB_JIT_CACHE (default ~/.cache/nnest_b200/jit), which the ranks of a run may share.  n_compiled_out (may
+ * be NULL) receives the number of variants this call compiled (0 when they came from either cache).  Needs a device of
+ * compute capability 10.0 and libnvrtc.so.12 (else NNB_ERR_UNSUPPORTED).  Synchronous.
+ */
+int nnb_set_user_likelihood(nnb_handle* h, const char* source, int* n_compiled_out);
+/*
+ * Compiles `source` as nnb_set_user_likelihood would, without a handle or a device: NNB_OK, or NNB_ERR_ARG when it does
+ * not compile (NNB_ERR_UNSUPPORTED without NVRTC).  log [host] (may be NULL) receives up to cap - 1 characters of NVRTC's
+ * log, NUL-terminated.
+ */
+int nnb_user_likelihood_check(const char* source, char* log, size_t cap);
 
 /*
  * logl[r] = safe_loglike(u[r]) for n rows (nnest/sampler.py:110-133): non-finite values become

@@ -9,14 +9,15 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, os.environ.get('NNB_LIB_DIR', 'lib'), 'libnnb.so')   # see build.py
 
-NNB_ABI_VERSION = 13
+NNB_ABI_VERSION = 14
 NNB_MAX_DIM = 128
 NNB_MAX_BLOCKS = 16
+NNB_MAX_LIKE_PARAMS = 160
 
 NNB_OK, NNB_ERR_ARG, NNB_ERR_CUDA, NNB_ERR_STATE, NNB_ERR_UNSUPPORTED, NNB_ERR_START = 0, -1, -2, -3, -4, -5
 NNB_FLOW_TRANSLATE_ONLY, NNB_FLOW_CONST_SCALE = 1, 2
 (NNB_LIKE_ROSENBROCK, NNB_LIKE_HIMMELBLAU, NNB_LIKE_GAUSSIAN, NNB_LIKE_EGGBOX, NNB_LIKE_GAUSSIAN_MIX,
- NNB_LIKE_GAUSSIAN_SHELL) = range(6)
+ NNB_LIKE_GAUSSIAN_SHELL, NNB_LIKE_USER) = range(7)
 NNB_PRIOR_NONE, NNB_PRIOR_BOX_U, NNB_PRIOR_BOX_V = 0, 1, 2
 NNB_MODE_HARD, NNB_MODE_MH = 0, 1
 NNB_IMPL_AUTO, NNB_IMPL_FFMA, NNB_IMPL_TCGEN05, NNB_IMPL_WARP = 0, 1, 2, 3
@@ -76,6 +77,8 @@ SYMBOLS = {
     'nnb_flow_forward': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
                                    C.c_void_p, C.c_int64, C.c_void_p]),
     'nnb_set_target': (C.c_int, [C.c_void_p, C.c_int, C.POINTER(nnb_target)]),
+    'nnb_set_user_likelihood': (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_int)]),
+    'nnb_user_likelihood_check': (C.c_int, [C.c_char_p, C.c_char_p, C.c_size_t]),
     'nnb_loglike': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
                               C.c_int64, C.c_void_p]),
     'nnb_mcmc_init': (C.c_int, [C.c_void_p, C.POINTER(nnb_mcmc_init_args), C.c_void_p]),
@@ -110,6 +113,27 @@ class NNBError(RuntimeError):
         self.code = code
 
 
+def _load_nvrtc():
+    """Make libnvrtc.so.12 visible to libnnb.so's dlopen (user likelihoods, nnb_jit.cu), from the first place that has
+    it: the loader's search path, torch's NVRTC wheel (12.8, which also targets sm_100a), $CUDA_HOME/lib64,
+    /usr/local/cuda/lib64.  Without it libnnb.so still loads; only user likelihoods are unavailable."""
+    candidates = ['libnvrtc.so.12']
+    try:
+        import nvidia.cuda_nvrtc
+        candidates.append(os.path.join(list(nvidia.cuda_nvrtc.__path__)[0], 'lib', 'libnvrtc.so.12'))
+    except Exception:
+        pass
+    if os.environ.get('CUDA_HOME'):
+        candidates.append(os.path.join(os.environ['CUDA_HOME'], 'lib64', 'libnvrtc.so.12'))
+    candidates.append('/usr/local/cuda/lib64/libnvrtc.so.12')
+    for path in candidates:
+        try:
+            return C.CDLL(path, mode=C.RTLD_GLOBAL)
+        except OSError:
+            continue
+    return None
+
+
 def load():
     """Load libnnb.so and set prototypes.  Raises if the library has not been built."""
     global _lib
@@ -126,6 +150,7 @@ def load():
                           '`python -m nnest_b200.build`', RuntimeWarning)
     except Exception:
         pass
+    _load_nvrtc()
     lib = C.CDLL(LIB_PATH)
     for name, (res, args) in SYMBOLS.items():
         fn = getattr(lib, name)      # AttributeError if the .so does not export a declared symbol

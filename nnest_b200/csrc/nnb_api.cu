@@ -85,6 +85,7 @@ extern "C" void nnb_destroy(nnb_handle* h) {
   if (h->d_stats_ws) cudaFree(h->d_stats_ws);
   if (h->d_nn_part) cudaFree(h->d_nn_part);
   if (h->d_nn_ws) cudaFree(h->d_nn_ws);
+  nnb_jit_free(h);
   delete h;
 }
 
@@ -176,6 +177,8 @@ extern "C" int nnb_set_flow(nnb_handle* h, int d, int hidden, int num_layers, in
 extern "C" int nnb_set_target(nnb_handle* h, int d, const nnb_target* t) {
   if (!h || !t) return NNB_ERR_ARG;
   if (d < 1 || d > NNB_MAX_DIM) return fail(h, NNB_ERR_ARG, "x_dim must be in [1, NNB_MAX_DIM]");
+  if (t->like_id == NNB_LIKE_USER && !h->jit)
+    return fail(h, NNB_ERR_STATE, "NNB_LIKE_USER: no user likelihood installed (nnb_set_user_likelihood)");
   if (t->n_like_params < 0 || t->n_like_params > NNB_MAX_LIKE_PARAMS || (t->n_like_params && !t->like_params))
     return fail(h, NNB_ERR_ARG, "bad likelihood parameter array");
   int need = 0;
@@ -194,7 +197,8 @@ extern "C" int nnb_set_target(nnb_handle* h, int d, const nnb_target* t) {
       }
       break;
     case NNB_LIKE_GAUSSIAN_SHELL: need = 2 + d; break;
-    default: return fail(h, NNB_ERR_UNSUPPORTED, "unknown likelihood id (arbitrary Python likelihoods cannot run on the device)");
+    case NNB_LIKE_USER: need = t->n_like_params; break;   // the user's source reads what it was given
+    default: return fail(h, NNB_ERR_UNSUPPORTED, "unknown likelihood id (Python likelihoods cannot run on the device: write it in CUDA C++, nnb_set_user_likelihood)");
   }
   if (t->n_like_params != need) return fail(h, NNB_ERR_ARG, "wrong number of likelihood parameters");
   if (t->prior_kind != NNB_PRIOR_NONE && (!t->prior_lo || !t->prior_hi))
@@ -271,13 +275,14 @@ extern "C" int nnb_loglike(nnb_handle* h, const void* u, int in_f64, int64_t u_r
   cudaStream_t st = (cudaStream_t)stream;
   size_t sm = smem_bytes(0, target_doubles(h->tdesc.d, h->tdesc.n_params), h->tdesc.d, 0);
   int grid = nnb_grid_for(h, n, 8);
-  if (in_f64)
-    loglike_kernel<double><<<grid, kBlockThreads, sm, st>>>(h->tdesc, h->d_target, (const double*)u, u_rs, u_cs, logl,
-                                                             logp, n);
-  else
-    loglike_kernel<float><<<grid, kBlockThreads, sm, st>>>(h->tdesc, h->d_target, (const float*)u, u_rs, u_cs, logl,
-                                                            logp, n);
-  NNB_CUDA(h, cudaGetLastError());
+  int rc = NNB_OK;
+  const void* fn = in_f64 ? nnb_kernel(h, (const void*)loglike_kernel<double>, &rc, "loglike_kernel<double>")
+                          : nnb_kernel(h, (const void*)loglike_kernel<float>, &rc, "loglike_kernel<float>");
+  if (!fn) return rc;
+  long long rs = u_rs, cs = u_cs, nn = n;
+  void* args[] = {(void*)&h->tdesc, (void*)&h->d_target, (void*)&u, (void*)&rs, (void*)&cs, (void*)&logl, (void*)&logp,
+                  (void*)&nn};
+  NNB_CUDA(h, cudaLaunchKernel(fn, dim3(grid), dim3(kBlockThreads), args, sm, st));
   return NNB_OK;
 }
 

@@ -7,9 +7,16 @@
 //                                                      nnest/sampler.py:100-163)
 // Layout conventions are described in DESIGN.md ("Data layout").
 #pragma once
+#ifndef __CUDACC_RTC__
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
+#else   // NVRTC (user likelihoods, nnb_jit.cu): no toolkit headers
+typedef unsigned int uint32_t;
+typedef unsigned long long uint64_t;
+typedef long long int64_t;
+#define INFINITY __int_as_float(0x7f800000)
+#endif
 
 #include "../../include/nnb.h"
 
@@ -456,6 +463,13 @@ __device__ __forceinline__ double loglike_T(const TargetSmem& tg, const XG& xg) 
       out = -((rad - rshell) * (rad - rshell)) / (2.0 * sigma * sigma);
       break;
     }
+#ifdef NNB_USER_LOGLIKE
+    case NNB_LIKE_USER: {  // the user's CUDA C++ (nnest_b200.likelihoods.CudaLikelihood), compiled in by nnb_jit.cu
+      out = nnb_user_loglike(v, d, tg.params);
+      f32_typed = sizeof(T) == 4;
+      break;
+    }
+#endif
     default:
       out = __longlong_as_double(0x7ff8000000000000LL);
   }

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <cstdio>
 #include <string>
 #include <vector>
 
@@ -54,6 +55,7 @@ struct nnb_handle {
   size_t nn_ws_floats = 0;
   int nn_part_cap = 0;
   double* d_stats_ws = nullptr;   // chain diagnostics (nnb_stats.cu)
+  struct nnb_jit_state* jit = nullptr;   // user likelihood and its compiled kernels (nnb_jit.cu)
   std::string err;
 };
 
@@ -63,6 +65,10 @@ int nnb_launch_mcmc_tc(nnb_handle* h, McmcParams p, int steps, cudaStream_t st);
 int nnb_warp_pack(nnb_handle* h, const float* weights_natural);                       // nnb_warp.cu
 int nnb_launch_mcmc_warp(nnb_handle* h, McmcParams p, int steps, cudaStream_t st, bool* ran);   // nnb_warp.cu
 long long nnb_warp_capacity(const nnb_handle* h);                                     // nnb_warp.cu
+void nnb_jit_free(nnb_handle* h);                                                      // nnb_jit.cu
+// the kernel `name` (a template instantiation, e.g. "mcmc_kernel<16, 0>") compiled around the handle's user likelihood;
+// nullptr with *rc set on failure
+const void* nnb_user_kernel(nnb_handle* h, const std::string& name, int* rc);          // nnb_jit.cu
 int nnb_spline_flow(nnb_handle* h, bool inverse, const float* in, int64_t irs, int64_t ics, float* out, int64_t ors,
                     int64_t ocs, float* logdet, int* empty_out, int64_t n, cudaStream_t st);      // nnb_spline.cu
 int nnb_spline_init(nnb_handle* h, const InitParams& p, cudaStream_t st);              // nnb_spline.cu
@@ -91,6 +97,17 @@ static inline cudaError_t nnb_reserve(T** ptr, size_t* cap, size_t need) {
 template <typename K>
 static inline cudaError_t nnb_set_smem(K kernel, size_t bytes) {
   return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
+
+// The kernel a launcher runs: `builtin` (the ahead-of-time instantiation), or with the user likelihood selected
+// (NNB_LIKE_USER) the same instantiation compiled by NVRTC around the user's source.  `fmt`/`args` spell the
+// instantiation, e.g. ("mcmc_kernel<%d, %d>", H, MODE).  nullptr with *rc set on failure.
+template <typename... A>
+static inline const void* nnb_kernel(nnb_handle* h, const void* builtin, int* rc, const char* fmt, A... args) {
+  if (h->tdesc.like_id != NNB_LIKE_USER) return builtin;
+  char name[128];
+  snprintf(name, sizeof(name), fmt, args...);
+  return nnb_user_kernel(h, name, rc);
 }
 
 static inline int nnb_grid_for(nnb_handle* h, long long n, int ctas_per_sm) {

@@ -6,6 +6,7 @@
 //   mcmc_init_kernel<H>       chain start                       (nnest/sampler.py:262-289)
 //   mcmc_kernel<H, MODE>      `steps` fused MCMC steps          (nnest/sampler.py:291-444)
 #pragma once
+#ifndef __CUDACC_RTC__
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -13,6 +14,7 @@
 #include <cstring>
 #include <string>
 #include <vector>
+#endif
 
 #include "nnb_device.cuh"
 

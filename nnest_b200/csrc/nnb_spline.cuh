@@ -21,7 +21,9 @@
 //   f2: W0[H*nup]  b0[H] W1[H*H] b1[H] W2[H*H] b2[H] W3[o2*H] b3[o2]     o2 = (3K-1) nlow   (conditioner of the lower half)
 // with nlow = d/2 (+1 when d is odd), nup = d - nlow; all matrices row-major (out, in) like nn.Linear.
 #pragma once
+#ifndef __CUDACC_RTC__
 #include <math.h>
+#endif
 
 #ifdef __CUDACC__
 #define NNB_HD __host__ __device__ __forceinline__

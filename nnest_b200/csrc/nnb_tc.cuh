@@ -11,8 +11,10 @@
 //     i.e. LBO (K direction) = nN * 128 B, SBO (N direction) = 128 B; successive K steps are 2*nN*128 B apart;
 //   * FP32 parity: every product is evaluated as 3xTF32 (a_hi*b_hi + a_lo*b_hi + a_hi*b_lo).
 #pragma once
+#ifndef __CUDACC_RTC__
 #include <cuda_runtime.h>
 #include <stdint.h>
+#endif
 
 namespace nnb {
 namespace tc {

@@ -1008,10 +1008,12 @@ mcmc_tc_kernel(TcFlowDesc f, const float* __restrict__ wglob, TargetDesc td, con
   if (warp == 0) tc::tmem_dealloc(*tmem_base_s, tmem_cols);
 }
 
+#ifndef __CUDACC_RTC__
 __host__ inline size_t tc_smem_bytes(const TcFlowDesc& f, int tdoubles, int ntiles, int npart) {
   return (size_t)f.total_floats * 4 + (size_t)tdoubles * 8 + 3 * (size_t)ntiles * f.d * 128 * 4 +
          (size_t)ntiles * (npart + 1) * 128 * 4 + (size_t)ntiles * 128 * 4 + 2 * kTcMaxTiles * 8 + 8 + 32 * 4 +
          NNB_MAX_BLOCKS * 8 + 8;
 }
+#endif
 
 }  // namespace nnb

@@ -17,6 +17,10 @@ static int launch_tc_mode(nnb_handle* h, McmcParams p, int steps, cudaStream_t s
   // block: +1.4 ms per cooperative launch).
   static_assert(sizeof(TcFlowDesc) + sizeof(TargetDesc) + sizeof(McmcParams) + sizeof(TcConsts) + 2 * sizeof(void*) + 32 <= 4096,
                 "kernel parameters of mcmc_tc_kernel exceed 4 KB");
+  int rc = NNB_OK;
+  const void* fn = nnb_kernel(h, (const void*)mcmc_tc_kernel<MODE, NPART, DD>, &rc, "nnb::mcmc_tc_kernel<%d, %d, %d>", MODE,
+                              NPART, DD);
+  if (!fn) return rc;
   TcConsts cst = h->tc_consts;
   {
     const int d = h->tcflow.d, t0 = tc_cb_off(d, h->tcflow.L, h->tcflow.B);
@@ -35,7 +39,7 @@ static int launch_tc_mode(nnb_handle* h, McmcParams p, int steps, cudaStream_t s
   size_t sm = tc_smem_bytes(h->tcflow, tdoubles, ntiles, NPART);
   const size_t one_cta_per_sm = 116 * 1024;   // TMEM is allocated per CTA: keep a single CTA resident per SM
   if (sm < one_cta_per_sm) sm = one_cta_per_sm;
-  NNB_CUDA(h, nnb_set_smem(mcmc_tc_kernel<MODE, NPART, DD>, sm));
+  NNB_CUDA(h, nnb_set_smem(fn, sm));
   const int grid = (int)((p.n + cpc - 1) / cpc);
   const int block = ntiles * 128 * NPART;   // fixed warp slots; a partial last tile leaves some idle
   p.cpc = (int)cpc;
@@ -52,6 +56,7 @@ static int launch_tc_mode(nnb_handle* h, McmcParams p, int steps, cudaStream_t s
   for (int j = 0; j < 4; ++j) p.tc_delay[j] = ntiles > 1 ? delays_env.v[j] : 0;
   // Persistent path: all steps in ONE cooperative launch (every CTA resident, one per SM), the global accept count
   // of each step travels through a grid barrier.  Needs grid <= SM count; otherwise one launch per step.
+  void* args[] = {(void*)&h->tcflow, (void*)&h->d_weights_tc, (void*)&h->tdesc, (void*)&h->d_target, (void*)&p, (void*)&cst};
   static const bool no_coop = getenv("NNB_NO_COOP") != nullptr;
   if (!no_coop && p.dynamic && h->coop_supported && grid <= h->sm_count && steps > 1) {
     if (h->step_counts_cap < steps) {
@@ -69,9 +74,7 @@ static int launch_tc_mode(nnb_handle* h, McmcParams p, int steps, cudaStream_t s
       tiles += (mine + 127) / 128;
     }
     p.total_tiles = (int)tiles;
-    void* args[] = {(void*)&h->tcflow, (void*)&h->d_weights_tc, (void*)&h->tdesc, (void*)&h->d_target, (void*)&p,
-                    (void*)&cst};
-    NNB_CUDA(h, cudaLaunchCooperativeKernel((const void*)mcmc_tc_kernel<MODE, NPART, DD>, dim3(grid), dim3(block), args, sm, st));
+    NNB_CUDA(h, cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(block), args, sm, st));
     h->last_launches = 1;
     return NNB_OK;
   }
@@ -79,13 +82,12 @@ static int launch_tc_mode(nnb_handle* h, McmcParams p, int steps, cudaStream_t s
   if (p.dynamic) {
     for (int s = 0; s < steps; ++s) {
       p.s0 = s; p.nsteps = 1;
-      mcmc_tc_kernel<MODE, NPART, DD><<<grid, block, sm, st>>>(h->tcflow, h->d_weights_tc, h->tdesc, h->d_target, p, cst);
+      NNB_CUDA(h, cudaLaunchKernel(fn, dim3(grid), dim3(block), args, sm, st));
     }
   } else {
     p.s0 = 0; p.nsteps = steps;
-    mcmc_tc_kernel<MODE, NPART, DD><<<grid, block, sm, st>>>(h->tcflow, h->d_weights_tc, h->tdesc, h->d_target, p, cst);
+    NNB_CUDA(h, cudaLaunchKernel(fn, dim3(grid), dim3(block), args, sm, st));
   }
-  NNB_CUDA(h, cudaGetLastError());
   h->last_launches = p.dynamic ? steps : 1;
   return NNB_OK;
 }

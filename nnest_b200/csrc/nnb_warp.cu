@@ -65,8 +65,7 @@ namespace {
 
 // chains per CTA and grid such that every CTA is resident (needed by the per-step grid barrier): spread the batch over
 // all SMs, two CTAs per SM at most (launch bounds); returns false when the batch does not fit
-template <int MODE, int DD>
-bool warp_plan(nnb_handle* h, long long n, int tdoubles, int* cpc_out, int* grid_out, size_t* smem_out) {
+bool warp_plan(nnb_handle* h, const void* fn, long long n, int tdoubles, int* cpc_out, int* grid_out, size_t* smem_out) {
   for (int per_sm = 1; per_sm <= 2; ++per_sm) {
     long long cpc = (n + (long long)h->sm_count * per_sm - 1) / ((long long)h->sm_count * per_sm);
     cpc = (cpc + 1) & ~1ll;              // whole warps
@@ -75,9 +74,8 @@ bool warp_plan(nnb_handle* h, long long n, int tdoubles, int* cpc_out, int* grid
     const size_t sm = warp_smem_bytes(h->warpflow, tdoubles, (int)cpc);
     if (sm * per_sm > (size_t)h->max_smem_per_sm || sm > (size_t)h->max_smem) continue;
     int occ = 0;
-    if (nnb_set_smem(mcmc_warp_kernel<MODE, DD>, sm) != cudaSuccess) continue;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mcmc_warp_kernel<MODE, DD>, (int)cpc * kWarpLanes, sm) !=
-        cudaSuccess)
+    if (nnb_set_smem(fn, sm) != cudaSuccess) continue;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, (int)cpc * kWarpLanes, sm) != cudaSuccess)
       continue;
     const long long grid = (n + cpc - 1) / cpc;
     if (grid > (long long)occ * h->sm_count) continue;
@@ -93,10 +91,14 @@ int launch_warp_mode(nnb_handle* h, McmcParams p, int steps, cudaStream_t st, bo
   int cpc = 0, grid = 0;
   size_t sm = 0;
   *ran = false;
-  if (!warp_plan<MODE, DD>(h, p.n, tdoubles, &cpc, &grid, &sm)) return NNB_OK;
+  int rc = NNB_OK;
+  const void* fn = nnb_kernel(h, (const void*)mcmc_warp_kernel<MODE, DD>, &rc, "nnb::mcmc_warp_kernel<%d, %d>", MODE, DD);
+  if (!fn) return rc;
+  if (!warp_plan(h, fn, p.n, tdoubles, &cpc, &grid, &sm)) return NNB_OK;
   if (p.dynamic && steps > 1 && !h->coop_supported) return NNB_OK;
   p.cpc = cpc;
   p.s0 = 0; p.nsteps = steps;
+  void* args[] = {(void*)&h->warpflow, (void*)&h->d_weights_warp, (void*)&h->tdesc, (void*)&h->d_target, (void*)&p};
   if (p.dynamic && steps > 1) {
     if (h->step_counts_cap < steps) {
       if (h->d_step_counts) cudaFree(h->d_step_counts);
@@ -106,17 +108,14 @@ int launch_warp_mode(nnb_handle* h, McmcParams p, int steps, cudaStream_t st, bo
     }
     NNB_CUDA(h, cudaMemsetAsync(h->d_step_counts, 0, sizeof(unsigned long long) * steps, st));
     p.coop = 1; p.step_counts = h->d_step_counts;
-    void* args[] = {(void*)&h->warpflow, (void*)&h->d_weights_warp, (void*)&h->tdesc, (void*)&h->d_target, (void*)&p};
-    NNB_CUDA(h, cudaLaunchCooperativeKernel((const void*)mcmc_warp_kernel<MODE, DD>, dim3(grid), dim3(cpc * kWarpLanes), args,
-                                            sm, st));
+    NNB_CUDA(h, cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(cpc * kWarpLanes), args, sm, st));
   } else if (p.dynamic) {
     // a single step: the scale update after it is the only one; run it through the cooperative path too when possible,
     // otherwise leave the batch to the other kernels
     return NNB_OK;
   } else {
     p.coop = 0; p.step_counts = nullptr;
-    mcmc_warp_kernel<MODE, DD><<<grid, cpc * kWarpLanes, sm, st>>>(h->warpflow, h->d_weights_warp, h->tdesc, h->d_target, p);
-    NNB_CUDA(h, cudaGetLastError());
+    NNB_CUDA(h, cudaLaunchKernel(fn, dim3(grid), dim3(cpc * kWarpLanes), args, sm, st));
   }
   h->last_launches = 1;
   *ran = true;

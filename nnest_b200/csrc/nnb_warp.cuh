@@ -43,9 +43,11 @@ __host__ __device__ inline int warp_chain_floats(int d) {
   const int c = 6 * round4(d) + 64;
   return (c & 31) == 16 ? c : ((c + 31) & ~31) + 16;
 }
+#ifndef __CUDACC_RTC__
 __host__ inline size_t warp_smem_bytes(const WarpFlowDesc& f, int tdoubles, int cpc) {
   return (size_t)f.total_floats * 4 + (size_t)((tdoubles + 1) & ~1) * 8 + (size_t)cpc * warp_chain_floats(f.d) * 4 + 64;
 }
+#endif
 
 __device__ __forceinline__ float warp_tanh(float x) {   // 1 - 2 / (e^{2x} + 1), MUFU ex2 / rcp (as tc_tanh)
   float e, rc;

@@ -281,8 +281,18 @@ class Engine(object):
         return acceptance, T / ess, jump_distance
 
     # ---- target -----------------------------------------------------------------------------
+    def set_user_likelihood(self, source):
+        """Install a CUDA C++ likelihood (nnb_set_user_likelihood): returns the number of kernel variants compiled."""
+        n = C.c_int(0)
+        self._check(self.lib.nnb_set_user_likelihood(self.h, source.encode(), C.byref(n)))
+        self.user_source = source
+        return n.value
+
     def set_target(self, d, like_id, like_params=(), t_scale=None, t_shift=None, compute_f64=False,
-                   prior_kind=L.NNB_PRIOR_NONE, prior_lo=None, prior_hi=None):
+                   prior_kind=L.NNB_PRIOR_NONE, prior_lo=None, prior_hi=None, user_source=None):
+        """user_source: CUDA C++ of the likelihood NNB_LIKE_USER selects, installed first when it is not the current one."""
+        if user_source is not None and user_source != getattr(self, 'user_source', None):
+            self.set_user_likelihood(user_source)
         t = L.nnb_target()
         keep = []
         t.like_id = like_id

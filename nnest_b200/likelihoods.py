@@ -34,6 +34,10 @@ class Likelihood(object):
     def device_params(self):
         return []
 
+    def device_source(self):
+        """CUDA C++ of a user likelihood (CudaLikelihood), None for the built-in ones."""
+        return None
+
     def __call__(self, x):
         """x: (n, x_dim) or (x_dim,) array in the likelihood's own coordinates -> log-likelihood(s)."""
         import torch
@@ -46,7 +50,7 @@ class Likelihood(object):
             xx = xx.astype(np.float64)
         self.num_evaluations += xx.shape[0]
         eng = _eval_engine()
-        eng.set_target(self.x_dim, self.like_id, self.device_params())
+        eng.set_target(self.x_dim, self.like_id, self.device_params(), user_source=self.device_source())
         out = eng.loglike(torch.from_numpy(xx).to(eng.device)).cpu().numpy()
         if self.follows_input_dtype and xx.dtype == np.float32:
             out = out.astype(np.float32)
@@ -178,3 +182,54 @@ class GaussianMix(Likelihood):
         p = np.zeros(self.x_dim)
         p[:2] = self.positions[int(np.argmax(self.weights))]
         return self(p)
+
+
+class CudaLikelihood(Likelihood):
+    """A likelihood written in CUDA C++, compiled at run time (NVRTC) into the library's own MCMC step kernels.
+
+    `source` defines
+
+        template <typename X>
+        __device__ double nnb_user_loglike(const X& x, int d, const double* params);
+
+    where x(i) is coordinate i of the point after the sampler's affine transform -- a float when the target computes in
+    float32 (float32 points, float32 transform), a double otherwise: `decltype(x(0))` names it -- and `params` holds the
+    `params` given here (at most NNB_MAX_LIKE_PARAMS doubles).  Larger constants, such as an inverse covariance, belong in
+    the source as __constant__ arrays.  A non-finite value is clamped as for the built-in likelihoods: to -inf when x(i)
+    is a float, to -1e100 otherwise.  Write float arithmetic with the *_rn intrinsics (__fadd_rn, __fmul_rn, ...) where
+    the exact rounding matters: the compiler contracts a * b + c into one fused multiply-add otherwise.
+
+    The source is compiled once here, without a device: a source that does not compile raises ValueError with the
+    compiler's log.  Compiled kernels are cached on disk under $NNB_JIT_CACHE (default ~/.cache/nnest_b200/jit).
+    """
+    like_id = L.NNB_LIKE_USER
+
+    def __init__(self, x_dim, source, params=(), max_loglike=None):
+        import ctypes as C
+        params = [float(p) for p in np.asarray(params, dtype=np.float64).ravel()]
+        if len(params) > L.NNB_MAX_LIKE_PARAMS:
+            raise ValueError('CudaLikelihood takes at most %d params, got %d' % (L.NNB_MAX_LIKE_PARAMS, len(params)))
+        if not isinstance(source, str):
+            raise ValueError('source must be a string of CUDA C++')
+        log = C.create_string_buffer(1 << 16)
+        rc = L.load().nnb_user_likelihood_check(source.encode(), log, len(log))
+        if rc == L.NNB_ERR_UNSUPPORTED:
+            raise RuntimeError('CudaLikelihood needs NVRTC (libnvrtc.so.12), which could not be loaded')
+        if rc != L.NNB_OK:
+            raise ValueError('the likelihood source does not compile:\n' + log.value.decode(errors='replace'))
+        self.source = source
+        self.params = params
+        self._max_loglike = max_loglike
+        super(CudaLikelihood, self).__init__(x_dim)
+
+    def device_params(self):
+        return list(self.params)
+
+    def device_source(self):
+        return self.source
+
+    @property
+    def max_loglike(self):
+        if self._max_loglike is None:
+            raise AttributeError('max_loglike was not given to CudaLikelihood')
+        return self._max_loglike

@@ -100,8 +100,8 @@ class Sampler(object):
         if not isinstance(loglike, Likelihood):
             raise NotImplementedError(
                 'loglike must be an instance of nnest_b200.likelihoods.* (Rosenbrock, Himmelblau, Gaussian, Eggbox, '
-                'GaussianMix, GaussianShell): arbitrary Python callables cannot run in the CUDA kernels and there is '
-                'no CPU fallback')
+                'GaussianMix, GaussianShell, or CudaLikelihood for your own likelihood written in CUDA C++): arbitrary '
+                'Python callables cannot run in the CUDA kernels and there is no CPU fallback')
         self._like = loglike
         self._user_transform = transform
         self._prior_obj = prior
@@ -210,7 +210,7 @@ class Sampler(object):
             lo, hi = prior.minimum.astype(np.float64), prior.maximum.astype(np.float64)
         self.engine.set_target(self.x_dim, self._like.like_id, self._like.device_params(), t_scale=self._t_scale,
                                t_shift=self._t_shift, compute_f64=self._t_f64, prior_kind=kind, prior_lo=lo,
-                               prior_hi=hi)
+                               prior_hi=hi, user_source=self._like.device_source())
 
     def _to_device_rows(self, x):
         if isinstance(x, list):
