@@ -35,6 +35,10 @@ extern "C" {
 #define NNB_MAX_DIM 128      /* x_dim */
 #define NNB_MAX_BLOCKS 16    /* num_blocks */
 #define NNB_MAX_LIKE_PARAMS 160
+/* derived parameters of a user likelihood (nnb_set_user_likelihood_derived).  The derived kernels hold them in a
+ * per-thread array of this many doubles: 32 doubles = 256 bytes a thread, which stays in registers / L1-resident local
+ * memory at 128 threads a CTA; more columns than this are better computed from the returned samples afterwards. */
+#define NNB_MAX_DERIVED 32
 
 enum {
   NNB_OK = 0,
@@ -172,6 +176,38 @@ int nnb_set_user_likelihood(nnb_handle* h, const char* source, int* n_compiled_o
  * log, NUL-terminated.
  */
 int nnb_user_likelihood_check(const char* source, char* log, size_t cap);
+
+/*
+ * Derived parameters of a user likelihood (the reference's `num_derived`: a likelihood returning (logl, derived)).
+ * With num_derived > 0 the source also defines
+ *     template <typename X> __device__ void nnb_user_derived(const X& x, int d, const double* params, double* derived);
+ * which writes derived[0 .. num_derived).  x and params mean what they mean for nnb_user_loglike, in the same arithmetic
+ * type; non-finite values are returned as they are (only the log-likelihood is clamped).
+ * nnb_set_user_likelihood_derived is nnb_set_user_likelihood that also compiles the derived kernels during the call, so a
+ * missing or wrong nnb_user_derived is refused here with NVRTC's log (NNB_ERR_ARG).  num_derived == 0 is exactly
+ * nnb_set_user_likelihood.  0 <= num_derived <= NNB_MAX_DERIVED, else NNB_ERR_ARG.
+ * nnb_user_likelihood_check_derived checks the same without a handle or a device, as nnb_user_likelihood_check does.
+ */
+int nnb_set_user_likelihood_derived(nnb_handle* h, const char* source, int num_derived, int* n_compiled_out);
+int nnb_user_likelihood_check_derived(const char* source, int num_derived, char* log, size_t cap);
+
+/*
+ * derived values of the target selected by nnb_set_target (like_id NNB_LIKE_USER with num_derived > 0, else
+ * NNB_ERR_STATE).  x(i) is formed from each row exactly as nnb_loglike and the step kernels form it, so derived values
+ * belong to the very point whose log-likelihood those report.
+ *   nnb_derived:       u [dev] n rows, float32 or float64 (in_f64), strides as nnb_loglike; out [dev] float64 (n, num_derived)
+ *                      row-major.
+ *   nnb_derived_trace: trace_x [dev] float32 (T, d, n) as nnb_mcmc_run writes it; evaluates the rows
+ *                      t_k = row0 + k * row_step, k < n_rows, into out [dev] float64 (n_rows, num_derived, n) chain-minor
+ *                      (element (k, j, c) at [(k * num_derived + j) * n + c]).  init [dev] float64 (num_derived, n) or
+ *                      NULL: when given, a chain whose point at t_k equals its row-0 point bit for bit in every
+ *                      coordinate gets init's values (the start's derived values the caller already has).
+ * Stream-ordered and asynchronous.
+ */
+int nnb_derived(nnb_handle* h, const void* u, int in_f64, int64_t u_rs, int64_t u_cs, double* out, int64_t n,
+                void* stream);
+int nnb_derived_trace(nnb_handle* h, const float* trace_x, int64_t n, int64_t row0, int64_t row_step, int64_t n_rows,
+                      const double* init, double* out, void* stream);
 
 /*
  * logl[r] = safe_loglike(u[r]) for n rows (nnest/sampler.py:110-133): non-finite values become

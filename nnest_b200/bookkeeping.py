@@ -13,10 +13,14 @@ from . import _lib as L
 
 
 class NSBook(object):
-    """State of the run: evidence, information, prior volume, iteration counter, dead points."""
+    """State of the run: evidence, information, prior volume, iteration counter, dead points.  With num_derived > 0 the
+    derived parameters of the dead points are kept too (saved_derived, next to saved_v), and the methods that move live
+    points take the live set's derived rows as well."""
 
-    def __init__(self, num_live_points):
+    def __init__(self, num_live_points, num_derived=0):
         self.nlive = int(num_live_points)
+        self.num_derived = int(num_derived)
+        self.saved_derived = []
         self.h = 0.0                                                      # nested.py:242-247
         self.logz = -1e300
         self.logvol = np.log(1.0 - np.exp(-1.0 / self.nlive))
@@ -53,11 +57,17 @@ class NSBook(object):
         out[m:] = active_v
         return out
 
+    def dead_derived(self):
+        """derived parameters (num_dead, num_derived) of the dead points, in the order of dead_points()"""
+        if not self.saved_derived:
+            return np.empty((0, self.num_derived))
+        return np.concatenate(self.saved_derived)
+
     def num_dead(self):
         return int(sum(len(a) for a in self.saved_logl))
 
     # ---- one iteration, exactly as the reference (used around refills / retrains / checkpoints) ---------------
-    def evidence_update(self, active_v, active_logl, worst):
+    def evidence_update(self, active_v, active_logl, worst, active_derived=None):
         """nested.py:273,280-293"""
         logwt = self.logvol + active_logl[worst]
         logz_new = np.logaddexp(self.logz, logwt)
@@ -67,6 +77,8 @@ class NSBook(object):
         self.saved_v.append(np.array(active_v[worst], copy=True)[None, :])
         self.saved_logwt.append(np.array([logwt]))
         self.saved_logl.append(np.array([active_logl[worst]]))
+        if self.num_derived:
+            self.saved_derived.append(np.array(active_derived[worst], dtype=np.float64)[None, :])
 
     def shrink(self, max_logl):
         """nested.py:460-464"""
@@ -77,12 +89,14 @@ class NSBook(object):
 
     # ---- a run of plain iterations ----------------------------------------------------------------------------
     def bulk(self, active_u, active_v, active_logl, transform, b_first, b_last, b_logl, nb, max_iters, dlogz,
-             it_limit):
+             it_limit, active_derived=None, b_derived=None):
         """Runs up to `max_iters` iterations that all start with accept_point == True (evidence update, scan of the
         batch from `nb`, replacement, shrink).  Mutates the live set and self.  Returns
         (nb, n_done, exhausted, finished): `exhausted` = the last started iteration used up the batch without
         finding a usable chain (its evidence update has been applied, accept_point is now False); `finished` = the
-        loop condition `fraction_remain > dlogz and it <= it_limit` (nested.py:269) failed after the last iteration."""
+        loop condition `fraction_remain > dlogz and it <= it_limit` (nested.py:269) failed after the last iteration.
+        With derived parameters, active_derived (nlive, num_derived) is updated like active_u, from b_derived (the derived
+        parameters of the rows of b_last), and the dead points' rows are recorded as for active_v."""
         lib = L.load()
         nlive, n_chains, d = self.nlive, b_first.shape[0], b_first.shape[1]
         worst = np.empty(max_iters + 1, dtype=np.int64)
@@ -147,6 +161,16 @@ class NSBook(object):
         rc = lib.nnb_ns_apply(ip(w), ip(pv), n_evid, n_done, d, dp(new_u), dp(new_v), dp(new_logl), dp(active_u),
                               dp(active_v), dp(active_logl), nlive, dp(dead))
         assert rc == 0, rc
+        if self.num_derived:
+            # the same rule as nnb_ns_apply's dead_out: the row that sat in slot worst[i] when iteration i started, i.e.
+            # the replacement an earlier iteration of this call wrote there (prev[i]) or the live row from before the call
+            new_der = b_derived[chain_c]
+            dead_der = np.where((pv >= 0)[:, None], new_der[np.maximum(pv, 0)] if n_done else 0.0, active_derived[w])
+            if n_done:                                              # the last write to a slot wins
+                _, first_rev = np.unique(w[:n_done][::-1], return_index=True)
+                keep = n_done - 1 - first_rev
+                active_derived[w[keep]] = new_der[keep]
+            self.saved_derived.append(dead_der)
         self.saved_v.append(dead)
         self.saved_logwt.append(np.array(logwt[:n_evid], copy=True))
         self.saved_logl.append(np.array(lstar[:n_evid], copy=True))

@@ -97,6 +97,7 @@ class Engine(object):
             raise L.NNBError(rc, (self.lib.nnb_last_error(None) or b'').decode())
         self.h = h
         self.d = None
+        self.num_derived = 0      # derived parameters of the installed user likelihood
         self.gpu_launches = 0     # kernels launched through this engine (bench.py reports it)
         self.default_impl = int(os.environ.get('NNB_IMPL', L.NNB_IMPL_AUTO))   # 0 auto, 1 ffma, 2 tcgen05
 
@@ -281,18 +282,25 @@ class Engine(object):
         return acceptance, T / ess, jump_distance
 
     # ---- target -----------------------------------------------------------------------------
-    def set_user_likelihood(self, source):
-        """Install a CUDA C++ likelihood (nnb_set_user_likelihood): returns the number of kernel variants compiled."""
+    def set_user_likelihood(self, source, num_derived=0):
+        """Install a CUDA C++ likelihood (nnb_set_user_likelihood, or nnb_set_user_likelihood_derived with num_derived > 0):
+        returns the number of kernel variants compiled."""
         n = C.c_int(0)
-        self._check(self.lib.nnb_set_user_likelihood(self.h, source.encode(), C.byref(n)))
+        if num_derived:
+            self._check(self.lib.nnb_set_user_likelihood_derived(self.h, source.encode(), int(num_derived), C.byref(n)))
+        else:
+            self._check(self.lib.nnb_set_user_likelihood(self.h, source.encode(), C.byref(n)))
         self.user_source = source
+        self.num_derived = int(num_derived)
         return n.value
 
     def set_target(self, d, like_id, like_params=(), t_scale=None, t_shift=None, compute_f64=False,
-                   prior_kind=L.NNB_PRIOR_NONE, prior_lo=None, prior_hi=None, user_source=None):
-        """user_source: CUDA C++ of the likelihood NNB_LIKE_USER selects, installed first when it is not the current one."""
-        if user_source is not None and user_source != getattr(self, 'user_source', None):
-            self.set_user_likelihood(user_source)
+                   prior_kind=L.NNB_PRIOR_NONE, prior_lo=None, prior_hi=None, user_source=None, num_derived=0):
+        """user_source: CUDA C++ of the likelihood NNB_LIKE_USER selects (with num_derived derived parameters), installed
+        first when it is not the current one."""
+        if user_source is not None and (user_source, num_derived) != (getattr(self, 'user_source', None),
+                                                                       getattr(self, 'num_derived', 0)):
+            self.set_user_likelihood(user_source, num_derived)
         t = L.nnb_target()
         keep = []
         t.like_id = like_id
@@ -327,6 +335,42 @@ class Engine(object):
                                              u.stride(1), _ptr(logl), _ptr(logp), n, _stream()))
             self.gpu_launches += 1
         return (logl, logp) if want_prior else logl
+
+    def derived(self, u, out=None):
+        """u (n,d) float32 or float64 cuda -> derived parameters float64 (n, num_derived) (nnb_derived)"""
+        assert u.is_cuda and u.dim() == 2 and u.shape[1] == self.target_d
+        assert u.dtype in (torch.float32, torch.float64)
+        n = u.shape[0]
+        if out is None:
+            out = torch.empty((n, self.num_derived), dtype=torch.float64, device=u.device)
+        assert out.dtype == torch.float64 and out.is_contiguous() and tuple(out.shape) == (n, self.num_derived)
+        if n:
+            self._check(self.lib.nnb_derived(self.h, _ptr(u), 1 if u.dtype == torch.float64 else 0, u.stride(0),
+                                             u.stride(1), _ptr(out), n, _stream()))
+            self.gpu_launches += 1
+        return out
+
+    def derived_trace(self, trace_x, row0=0, row_step=1, n_rows=None, init=None, out=None):
+        """Derived parameters of rows row0, row0 + row_step, ... (n_rows of them; default: to the end) of a device trace
+        float32 (T, d, n) -> float64 (n_rows, num_derived, n) (nnb_derived_trace).  init (num_derived, n) float64 cuda: the
+        values of chains that have not moved since row 0."""
+        assert trace_x.is_cuda and trace_x.dtype == torch.float32 and trace_x.is_contiguous() and trace_x.dim() == 3
+        T, d, n = trace_x.shape
+        assert d == self.target_d
+        if n_rows is None:
+            n_rows = len(range(row0, T, row_step))
+        assert n_rows == 0 or row0 + (n_rows - 1) * row_step < T
+        if out is None:
+            out = torch.empty((n_rows, self.num_derived, n), dtype=torch.float64, device=trace_x.device)
+        assert out.dtype == torch.float64 and out.is_contiguous() and tuple(out.shape) == (n_rows, self.num_derived, n)
+        if init is not None:
+            assert init.is_cuda and init.dtype == torch.float64 and init.is_contiguous() \
+                and tuple(init.shape) == (self.num_derived, n)
+        if n and n_rows:
+            self._check(self.lib.nnb_derived_trace(self.h, _ptr(trace_x), n, row0, row_step, n_rows, _ptr(init),
+                                                   _ptr(out), _stream()))
+            self.gpu_launches += 1
+        return out
 
     # ---- MCMC -------------------------------------------------------------------------------
     def mcmc_init(self, n, init_u=None, init_z=None, init_logl=None, seed=0, chain_offset=0, start_try=0,

@@ -50,10 +50,15 @@ class Likelihood(object):
             xx = xx.astype(np.float64)
         self.num_evaluations += xx.shape[0]
         eng = _eval_engine()
-        eng.set_target(self.x_dim, self.like_id, self.device_params(), user_source=self.device_source())
-        out = eng.loglike(torch.from_numpy(xx).to(eng.device)).cpu().numpy()
+        eng.set_target(self.x_dim, self.like_id, self.device_params(), user_source=self.device_source(),
+                       num_derived=self.num_derived)
+        xd = torch.from_numpy(xx).to(eng.device)
+        out = eng.loglike(xd).cpu().numpy()
         if self.follows_input_dtype and xx.dtype == np.float32:
             out = out.astype(np.float32)
+        if self.num_derived:
+            der = eng.derived(xd).cpu().numpy()
+            return (out[0], der[0]) if single else (out, der)
         return out[0] if single else out
 
     def loglike(self, x):
@@ -196,7 +201,18 @@ class CudaLikelihood(Likelihood):
     float32 (float32 points, float32 transform), a double otherwise: `decltype(x(0))` names it -- and `params` holds the
     `params` given here (at most NNB_MAX_LIKE_PARAMS doubles).  Larger constants, such as an inverse covariance, belong in
     the source as __constant__ arrays.  A non-finite value is clamped as for the built-in likelihoods: to -inf when x(i)
-    is a float, to -1e100 otherwise.  Write float arithmetic with the *_rn intrinsics (__fadd_rn, __fmul_rn, ...) where
+    is a float, to -1e100 otherwise.
+
+    num_derived > 0 (at most NNB_MAX_DERIVED): the source also defines
+
+        template <typename X>
+        __device__ void nnb_user_derived(const X& x, int d, const double* params, double* derived);
+
+    which writes derived[0 .. num_derived) at the point x -- the same x, in the same arithmetic type, as
+    nnb_user_loglike sees there; helper functions can be shared between the two.  Derived values are returned as they are
+    (no clamp), and they are not likelihood calls: the samplers evaluate them on the points they return, not on every
+    proposal.  Calling the likelihood then returns (logl, derived), as a likelihood with derived parameters does in the
+    reference.  Write float arithmetic with the *_rn intrinsics (__fadd_rn, __fmul_rn, ...) where
     the exact rounding matters: the compiler contracts a * b + c into one fused multiply-add otherwise.
 
     The source is compiled once here, without a device: a source that does not compile raises ValueError with the
@@ -204,20 +220,23 @@ class CudaLikelihood(Likelihood):
     """
     like_id = L.NNB_LIKE_USER
 
-    def __init__(self, x_dim, source, params=(), max_loglike=None):
+    def __init__(self, x_dim, source, params=(), max_loglike=None, num_derived=0):
         import ctypes as C
         params = [float(p) for p in np.asarray(params, dtype=np.float64).ravel()]
         if len(params) > L.NNB_MAX_LIKE_PARAMS:
             raise ValueError('CudaLikelihood takes at most %d params, got %d' % (L.NNB_MAX_LIKE_PARAMS, len(params)))
         if not isinstance(source, str):
             raise ValueError('source must be a string of CUDA C++')
+        if int(num_derived) != num_derived or not 0 <= num_derived <= L.NNB_MAX_DERIVED:
+            raise ValueError('num_derived must be an integer in [0, %d], got %r' % (L.NNB_MAX_DERIVED, num_derived))
         log = C.create_string_buffer(1 << 16)
-        rc = L.load().nnb_user_likelihood_check(source.encode(), log, len(log))
+        rc = L.load().nnb_user_likelihood_check_derived(source.encode(), int(num_derived), log, len(log))
         if rc == L.NNB_ERR_UNSUPPORTED:
             raise RuntimeError('CudaLikelihood needs NVRTC (libnvrtc.so.12), which could not be loaded')
         if rc != L.NNB_OK:
             raise ValueError('the likelihood source does not compile:\n' + log.value.decode(errors='replace'))
         self.source = source
+        self.num_derived = int(num_derived)
         self.params = params
         self._max_loglike = max_loglike
         super(CudaLikelihood, self).__init__(x_dim)

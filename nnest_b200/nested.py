@@ -146,7 +146,7 @@ class NestedSampler(Sampler):
             for f in glob.glob(os.path.join(self.logs['checkpoint'], 'checkpoint_*.txt')):
                 it = max(it, int(f.split('/checkpoint_')[1].split('.txt')[0]))
 
-        bk = NSBook(nlive)
+        bk = NSBook(nlive, self.num_derived)
         if it >= 0:
             if primary:
                 self.logger.info('Using checkpoint [%d]' % it)
@@ -166,6 +166,8 @@ class NestedSampler(Sampler):
                 bk.saved_v = [np.load(os.path.join(ckpt, 'saved_v.npy')).reshape(it, self.x_dim)]
                 bk.saved_logl = [np.load(os.path.join(ckpt, 'saved_logl.npy'))]
                 bk.saved_logwt = [np.load(os.path.join(ckpt, 'saved_logwt.npy'))]
+                if self.num_derived:
+                    bk.saved_derived = [np.load(os.path.join(ckpt, 'saved_derived.npy')).reshape(it, self.num_derived)]
             assert it == bk.num_dead()
             total_calls = data['ncall']
         else:
@@ -179,7 +181,7 @@ class NestedSampler(Sampler):
                 lo, hi = dist.shard_bounds(nlive, self.mpi_rank, self.mpi_size)
                 part, _ = self.loglike(active_u[lo:hi])
                 active_logl = dist.allgather_ragged(np.asarray(part, dtype=np.float64), nlive, self.device)
-                active_derived = np.empty((nlive, 0))
+                active_derived = self._derived_rows(active_u)      # every rank, all rows: no collective
                 total_calls = dist.allreduce_sum_int(self.total_calls, self.device)
             else:
                 active_logl, active_derived = self.loglike(active_u)
@@ -191,6 +193,7 @@ class NestedSampler(Sampler):
         active_u = np.ascontiguousarray(active_u, dtype=np.float64)
         active_v = np.ascontiguousarray(active_v, dtype=np.float64)
         active_logl = np.ascontiguousarray(active_logl, dtype=np.float64)
+        active_derived = np.ascontiguousarray(active_derived, dtype=np.float64).reshape(nlive, self.num_derived)
 
         lib = L.load()
         # Device-resident live set (float64, like the host arrays): chain starts are gathered from it on the device, and the
@@ -226,7 +229,8 @@ class NestedSampler(Sampler):
         scale = step_size
         batch = None
         samples = loglikes = None
-        b_first = b_last = b_logl = None
+        b_first = b_last = b_logl = b_derived = None
+        s_derived = None
         max_logl = np.max(active_logl)
 
         def next_special(i):
@@ -242,7 +246,8 @@ class NestedSampler(Sampler):
                 kmax = min(next_special(bk.it) - bk.it, 1 << 20)
                 if kmax > 0:
                     nb, n_done, exhausted, finished = bk.bulk(active_u, active_v, active_logl, self.transform, b_first,
-                                                              b_last, b_logl, nb, kmax, dlogz, max_iters)
+                                                              b_last, b_logl, nb, kmax, dlogz, max_iters,
+                                                              active_derived=active_derived, b_derived=b_derived)
                     if n_done:
                         max_logl = np.max(active_logl)
                         pend_slots.append(bk.last_slots)
@@ -262,7 +267,7 @@ class NestedSampler(Sampler):
             expected_vol = np.exp(-it / nlive)
 
             if accept_point:                                   # nested.py:280-293
-                bk.evidence_update(active_v, active_logl, worst)
+                bk.evidence_update(active_v, active_logl, worst, active_derived)
                 accept_point = False
 
             old_method = current_method
@@ -290,15 +295,16 @@ class NestedSampler(Sampler):
                 if get_samples:                                 # nested.py:316-377
                     nb = 0
                     if current_method == 'rejection_prior':
-                        samples, loglikes, _, nc = self._rejection_prior_sample(loglstar, num_trials=rejection_trials)
+                        samples, loglikes, s_derived, nc = self._rejection_prior_sample(loglstar,
+                                                                                        num_trials=rejection_trials)
                         label = 'Rejection prior'
                     elif current_method == 'rejection_flow':
-                        samples, loglikes, _, nc = self._rejection_flow_sample(
+                        samples, loglikes, s_derived, nc = self._rejection_flow_sample(
                             active_u, loglstar, enlargement_factor=rejection_enlargement_factor,
                             cache=it % rejection_cache_interval == 0 or it % update_interval == 0)
                         label = 'Rejection flow'
                     else:
-                        samples, loglikes, _, nc = self._density_sample(loglstar)
+                        samples, loglikes, s_derived, nc = self._density_sample(loglstar)
                         label = 'Density flow'
                     ncs.append(nc)
                     mean_calls = np.mean(ncs[-20:]) if len(ncs) > 20 else 0
@@ -313,10 +319,14 @@ class NestedSampler(Sampler):
                         # nested.py:295-298,366-377: every rank contributes its draw(s), all ranks consume the rank-ordered
                         # concatenation; a strategy expired on any rank is expired on all of them (every rank reaches
                         # this point in the same iteration, so the union is taken where the flag can change)
+                        drawn_dtype = np.asarray(samples).dtype
                         samples = dist.allgather_rows(torch.from_numpy(np.ascontiguousarray(
                             samples, dtype=np.float64)).to(self.device)).cpu().numpy()
                         loglikes = dist.allgather_rows(torch.from_numpy(np.ascontiguousarray(
                             loglikes, dtype=np.float64)).to(self.device)).cpu().numpy()
+                        # derived parameters of the gathered draws, on every rank, from the draws in the type they were
+                        # evaluated in (float32 flow draws travel as exact float64)
+                        s_derived = self._derived_rows(samples.astype(drawn_dtype))
                         expire = bool(dist.allreduce_sum_int(int(expire), self.device))
                         total_calls = dist.allreduce_sum_int(self.total_calls, self.device)
                     if expire:
@@ -331,6 +341,7 @@ class NestedSampler(Sampler):
                         active_u[worst] = samples[nb - 1, :]
                         active_v[worst] = self.transform(active_u[worst])
                         active_logl[worst] = loglikes[nb - 1]
+                        active_derived[worst] = s_derived[nb - 1]
                         live_dev = None                  # replaced on the host only: the device copy is rebuilt when needed
                         accept_point = True
                         break
@@ -356,6 +367,7 @@ class NestedSampler(Sampler):
                     batch = self._mcmc_refill(mcmc_steps, None, None, loglstar, step_size, mcmc_dynamic_step_size,
                                               keep_trace=chain_stats, live=(live_dev[0], live_dev[1], idx))
                     b_first, b_last, b_logl = self._refill_to_host(batch)     # all ranks' chains, rank order
+                    b_derived = self.refill_derived
                     total_calls = dist.allreduce_sum_int(self.total_calls, self.device) if self.use_mpi \
                         else self.total_calls
                     scale = batch['scale']
@@ -378,6 +390,8 @@ class NestedSampler(Sampler):
                     active_u[worst] = b_last[ib, :]
                     active_v[worst] = self.transform(active_u[worst])
                     active_logl[worst] = b_logl[ib]
+                    if self.num_derived:
+                        active_derived[worst] = b_derived[ib]
                     accept_point = True
                     pend_slots.append(np.array([worst], dtype=np.int64))
                     pend_chains.append(np.array([ib], dtype=np.int64))
@@ -414,7 +428,8 @@ class NestedSampler(Sampler):
                                            expired_strategies)
                     self.samples, self.loglikes, logwt = bk.dead_points()
                     self.weights = np.exp(logwt - bk.logz)
-                    self._save_samples(self.samples, self.loglikes, weights=self.weights)
+                    self._save_samples(self.samples, self.loglikes, weights=self.weights,
+                                       derived_samples=bk.dead_derived() if self.num_derived else None)
 
         saved_logl = np.concatenate(bk.saved_logl) if bk.saved_logl else np.empty((0,))
         saved_logwt = np.concatenate(bk.saved_logwt) if bk.saved_logwt else np.empty((0,))
@@ -438,14 +453,17 @@ class NestedSampler(Sampler):
         self.samples = bk.samples_with(active_v)        # dead points followed by the remaining live points
         self.weights = np.exp(np.concatenate((saved_logwt, fin_logwt)) - logz)
         self.loglikes = np.concatenate((saved_logl, active_logl))
-        self.active_u, self.active_logl = active_u, active_logl
+        self.active_u, self.active_logl, self.active_derived = active_u, active_logl, active_derived
+        # derived parameters of self.samples, row for row (None without them): the chain files carry them for the dead
+        # points too, an extension -- the reference saves none for its dead points
+        self.derived_samples = np.concatenate((bk.dead_derived(), active_derived)) if self.num_derived else None
 
         if primary:
             with open(os.path.join(self.logs['results'], 'final.csv'), 'w') as f:
                 writer = csv.writer(f)
                 writer.writerow(['niter', 'ncall', 'logz', 'logzerr', 'h'])
                 writer.writerow([it + 1, total_calls, logz, np.sqrt(h / nlive), h])
-            self._save_samples(self.samples, self.loglikes, weights=self.weights)
+            self._save_samples(self.samples, self.loglikes, weights=self.weights, derived_samples=self.derived_samples)
             self.logger.info("niter: {:d}\n ncall: {:d}\n nsamples: {:d}\n logz: {:6.3f} +/- {:6.3f}\n h: {:6.3f}"
                              .format(it + 1, int(total_calls), len(self.loglikes), logz, np.sqrt(h / nlive), h))
         # run diagnostics (NOT part of the reference's layout: only on request): one row per MCMC refill / flow fit
@@ -472,6 +490,8 @@ class NestedSampler(Sampler):
         np.save(os.path.join(ckpt, 'saved_v.npy'), saved_v if len(saved_logl) else [])
         np.save(os.path.join(ckpt, 'saved_logl.npy'), saved_logl)
         np.save(os.path.join(ckpt, 'saved_logwt.npy'), saved_logwt)
+        if self.num_derived:     # derived parameters of the dead points (not in the reference, which saves none)
+            np.save(os.path.join(ckpt, 'saved_derived.npy'), bk.dead_derived())
         with open(os.path.join(ckpt, 'checkpoint_%s.txt' % it), 'w') as f:
             json.dump({'logz': float(bk.logz), 'h': float(bk.h), 'logvol': float(bk.logvol), 'ncall': int(total_calls),
                        'fraction_remain': float(bk.fraction_remain), 'strategy': strategy,

@@ -23,7 +23,7 @@ import torch
 
 from . import _lib as L
 from . import dist
-from .likelihoods import Likelihood
+from .likelihoods import CudaLikelihood, Likelihood
 from .priors import UniformPrior
 from .trainer import Trainer
 from .utils.evaluation import acceptance_rate, effective_sample_size, mean_jump_distance
@@ -88,8 +88,14 @@ class Sampler(object):
         assert x_dim > num_slow
         if num_slow != 0:
             raise NotImplementedError('fast/slow hierarchies (num_slow > 0) are not on the accelerated path')
-        if num_derived != 0:
-            raise NotImplementedError('derived parameters need a Python likelihood; the device likelihoods have none')
+        # derived parameters come from the likelihood's own CUDA C++ (CudaLikelihood(num_derived=...)); checked before
+        # any device work, so a wrong combination fails fast
+        if num_derived != 0 and not isinstance(loglike, CudaLikelihood):
+            raise NotImplementedError('derived parameters (num_derived > 0) need a CudaLikelihood whose source defines '
+                                      'nnb_user_derived; the built-in likelihoods have none')
+        if isinstance(loglike, Likelihood) and loglike.num_derived != num_derived:
+            raise ValueError('num_derived=%d does not match the likelihood, which has %d derived parameters'
+                             % (num_derived, loglike.num_derived))
         self.num_slow = num_slow
         self.num_fast = x_dim - num_slow
         self.param_names = param_names
@@ -210,7 +216,7 @@ class Sampler(object):
             lo, hi = prior.minimum.astype(np.float64), prior.maximum.astype(np.float64)
         self.engine.set_target(self.x_dim, self._like.like_id, self._like.device_params(), t_scale=self._t_scale,
                                t_shift=self._t_shift, compute_f64=self._t_f64, prior_kind=kind, prior_lo=lo,
-                               prior_hi=hi, user_source=self._like.device_source())
+                               prior_hi=hi, user_source=self._like.device_source(), num_derived=self.num_derived)
 
     def _to_device_rows(self, x):
         if isinstance(x, list):
@@ -225,13 +231,24 @@ class Sampler(object):
 
     def loglike(self, x):
         """safe_loglike (nnest/sampler.py:110-133): loglike(transform(x)) for a batch of points in the flow's
-        coordinates, non-finite -> -1e100, call counter updated.  Returns (logl, derived (n, 0))."""
+        coordinates, non-finite -> -1e100, call counter updated.  Returns (logl, derived (n, num_derived)); derived values
+        are not counted as calls."""
         x, xd = self._to_device_rows(x)
         logl = self.engine.loglike(xd).cpu().numpy()
         self.total_calls += x.shape[0]
         if self._like.follows_input_dtype and x.dtype == np.float32 and not self._t_f64:
             logl = logl.astype(np.float32)
-        return logl, np.empty((x.shape[0], 0))
+        return logl, self._derived_rows(xd)
+
+    def _derived_rows(self, x):
+        """Derived parameters (n, num_derived) float64 of rows x (host array or cuda tensor, float32 or float64), evaluated
+        in the arithmetic the likelihood uses for rows of that type (nnb_derived); (n, 0) without derived parameters."""
+        n = x.shape[0] if x.ndim > 1 else 1
+        if not self.num_derived:
+            return np.empty((n, 0))
+        if not isinstance(x, torch.Tensor):
+            _, x = self._to_device_rows(x)
+        return self.engine.derived(x).cpu().numpy()
 
     def prior(self, x):
         """safe_prior (nnest/sampler.py:143-163): 0 inside the box, -inf outside."""
@@ -340,7 +357,11 @@ class Sampler(object):
         The arrays are host views of the chain-minor device trace (no extra transposition pass).
         Extensions (both default to the reference's behaviour): thin=k returns every k-th state of the trace (rows 0, k,
         2k, ...: arrays shaped (N, S//k+1, .)); sample_affine=(scale, shift) returns samples * scale + shift in float64,
-        evaluated on the device (what MCMCSampler.run applies to the whole trace on the host, mcmc.py:117)."""
+        evaluated on the device (what MCMCSampler.run applies to the whole trace on the host, mcmc.py:117).
+        With derived parameters `derived` is (N, S//k+1, num_derived) float64: row t is the derived values of the state
+        x_t, evaluated on the device for the returned rows only.  Given init_samples and init_derived (N, num_derived),
+        row 0 and every later row whose state is still bit-equal to row 0 hold init_derived, as the reference keeps the
+        start's values until the chain first moves."""
         if prior_volume_steps != 1:
             raise NotImplementedError('prior_volume_steps != 1')
         st, out, ncall = self._mcmc_device(mcmc_steps, step_size, dynamic_step_size, num_chains, init_samples,
@@ -349,28 +370,44 @@ class Sampler(object):
         samples = self._trace_to_host(out['trace_x'], rows, sample_affine).transpose(2, 0, 1)   # (T,d,N) -> (N,T,d) view
         latent_samples = self._trace_to_host(out['trace_z'], rows, None).transpose(2, 0, 1)
         loglikes = self._trace_to_host(out['trace_logl'], rows, None).transpose(1, 0)
-        derived_samples = np.empty((st.n, len(rows), 0))
+        init_der = None
+        if self.num_derived and init_samples is not None and init_derived is not None:
+            init_der = torch.from_numpy(np.ascontiguousarray(
+                np.asarray(init_derived, dtype=np.float64).reshape(st.n, self.num_derived).T)).to(self.device)
+        if self.num_derived:
+            derived_samples = self._trace_to_host(out['trace_x'], rows, None, derived_init=(init_der,)).transpose(2, 0, 1)
+        else:
+            derived_samples = np.empty((st.n, len(rows), 0))
         self._device_trace = out['trace_x']          # (S+1, d, N) on the device, for the chain statistics
         ts, tb = self._affine()
         for it in range(1, mcmc_steps + 1):
             if output_interval is not None and it % output_interval == 0:
                 full = out['trace_x'][:it + 1].cpu().numpy().transpose(2, 0, 1)
+                der = None
+                if self.num_derived:
+                    der = self.engine.derived_trace(out['trace_x'], 0, 1, it + 1, init=init_der).cpu().numpy()
+                    der = der.transpose(2, 0, 1)
                 self._save_samples(self.transform(full.reshape(-1, self.x_dim)).reshape(st.n, it + 1, self.x_dim),
-                                   out['trace_logl'][:it + 1].cpu().numpy().transpose(1, 0))
+                                   out['trace_logl'][:it + 1].cpu().numpy().transpose(1, 0), derived_samples=der)
             if stats_interval is not None and it % stats_interval == 0:
                 self._chain_stats(None, step=it, trace=self._device_trace, t_scale=ts, t_shift=tb)
         return samples, latent_samples, derived_samples, loglikes, out['scale'], ncall
 
     _STAGE_BYTES = 128 << 20
 
-    def _trace_to_host(self, trace, rows, affine):
+    def _trace_to_host(self, trace, rows, affine, derived_init=None):
         """Rows `rows` of a device trace (T, d, N) / (T, N) -> pageable host array (len(rows), ...), through two pinned
         staging buffers: the device->host copy of chunk k+1 runs while chunk k is moved into the result by a few host
         threads (a single pageable .cpu() of a multi-GB trace is bound by first-touch page faults on one core).
-        affine=(scale, shift): float64 rows * scale[:, None] + shift[:, None], computed on the device."""
+        affine=(scale, shift): float64 rows * scale[:, None] + shift[:, None], computed on the device.
+        derived_init=(init,): the derived parameters (len(rows), num_derived, N) float64 of the rows of the trace x
+        (T, d, N) instead, evaluated chunk by chunk (nnb_derived_trace; init: Engine.derived_trace), so that the full
+        derived trace never sits on the device."""
         from concurrent.futures import ThreadPoolExecutor
         inner = tuple(trace.shape[1:])
-        dtype = torch.float64 if affine is not None else trace.dtype
+        if derived_init is not None:
+            inner = (self.num_derived, trace.shape[2])
+        dtype = torch.float64 if affine is not None or derived_init is not None else trace.dtype
         out = np.empty((len(rows),) + inner, dtype=np.float64 if dtype == torch.float64 else np.float32)
         if not rows:
             return out
@@ -386,7 +423,10 @@ class Sampler(object):
 
         def launch(ci):
             a, b = chunks[ci]
-            src = trace[rows[a]:rows[b - 1] + 1:step]
+            if derived_init is not None:
+                src = self.engine.derived_trace(trace, rows[a], step, b - a, init=derived_init[0])
+            else:
+                src = trace[rows[a]:rows[b - 1] + 1:step]
             if affine is not None:
                 src = src.double() * sc[:, None] + sh[:, None]
             stage[ci % 2][:b - a].copy_(src, non_blocking=True)
@@ -443,6 +483,13 @@ class Sampler(object):
             host.copy_(t, non_blocking=True)
             out[key] = host
         self._gathered_dev = dev          # device copies of the gathered batch: source of the live-set updates
+        self.refill_derived = None
+        if self.num_derived:
+            # every rank evaluates the derived parameters of the gathered end states itself: the kernel is deterministic,
+            # so the ranks agree bit for bit without another collective
+            host = self._pinned('derived_last', (dev['last'].shape[0], self.num_derived), torch.float64)
+            host.copy_(self.engine.derived(dev['last']), non_blocking=True)
+            self.refill_derived = host.numpy()
         torch.cuda.current_stream().synchronize()
         return out['first'].numpy(), out['last'].numpy(), out['logl_last'].numpy()
 
@@ -524,7 +571,6 @@ class Sampler(object):
     def _rejection_prior_sample(self, loglstar, num_trials=None):
         """nnest/sampler.py:529-543.  num_trials=None: k prior draws per launch; np.random is then rewound and advanced
         by exactly the draws the one-at-a-time loop would have consumed, so a seeded run sees the same stream."""
-        derived = np.empty((1, 0))
         if num_trials is None:
             ncall = 0
             k = int(min(max(8, 2 * getattr(self, '_rej_prior_mean', 4)), 1 << 16))
@@ -542,7 +588,7 @@ class Sampler(object):
                     ncall += j + 1
                     self.total_calls += j + 1
                     self._rej_prior_mean = 0.8 * getattr(self, '_rej_prior_mean', 4) + 0.2 * ncall
-                    return x[j:j + 1], logl[j:j + 1], derived, ncall
+                    return x[j:j + 1], logl[j:j + 1], self._derived_rows(x[j:j + 1]), ncall
                 ncall += x.shape[0]
                 self.total_calls += x.shape[0]
                 k = min(2 * k, 1 << 16)
@@ -590,7 +636,7 @@ class Sampler(object):
                 lj = logl[j:j + 1].cpu().numpy()
                 if self._like.follows_input_dtype and not self._t_f64:
                     lj = lj.astype(np.float32)
-                return x[j:j + 1].cpu().numpy(), lj, np.empty((1, 0)), ncall
+                return x[j:j + 1].cpu().numpy(), lj, self._derived_rows(x[j:j + 1]), ncall
             n_eval = int(evaluated.sum())
             ncall += n_eval
             self.total_calls += n_eval
@@ -617,7 +663,7 @@ class Sampler(object):
                 lj = logl[j:j + 1].cpu().numpy()
                 if self._like.follows_input_dtype and not self._t_f64:
                     lj = lj.astype(np.float32)
-                return x[j:j + 1].cpu().numpy(), lj, np.empty((1, 0)), ncall
+                return x[j:j + 1].cpu().numpy(), lj, self._derived_rows(x[j:j + 1]), ncall
             n_eval = int(inside.sum())
             ncall += n_eval
             self.total_calls += n_eval
