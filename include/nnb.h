@@ -210,6 +210,45 @@ int nnb_derived_trace(nnb_handle* h, const float* trace_x, int64_t n, int64_t ro
                       const double* init, double* out, void* stream);
 
 /*
+ * A prior transform written by the user in CUDA C++ (the reference's `transform` callable, nnest/sampler.py:100-108,
+ * when it is not the affine map of t_scale / t_shift).  `source` defines
+ *     template <typename U> __device__ auto nnb_user_transform(const U& u, int i, int d, const double* params)
+ *         -> decltype(u(0));
+ * which returns coordinate i of v = transform(u).  u(j) is coordinate j of the unit-box point in the arithmetic type of
+ * the target (float when compute_f64 == 0 and the input is float32, double otherwise); any u(j) may be read, so
+ * transforms that mix coordinates are allowed.  v is not stored: every x(i) the likelihood, the BOX_V prior or the derived
+ * parameters read evaluates the transform once.  params are the transform_params given to nnb_set_target_user_transform.
+ * nnb_set_user_transform installs the source on the handle and compiles the likelihood kernels around it during the call
+ * (NNB_ERR_ARG with NVRTC's log in nnb_last_error when it does not compile); it compiles, caches and needs what
+ * nnb_set_user_likelihood does, and the two sources may be installed together.  n_compiled_out as there.  Synchronous.
+ * nnb_user_transform_check compiles `source` without a handle or a device, as nnb_user_likelihood_check does.
+ */
+int nnb_set_user_transform(nnb_handle* h, const char* source, int* n_compiled_out);
+int nnb_user_transform_check(const char* source, char* log, size_t cap);
+
+/*
+ * nnb_set_target with the installed user transform in place of the affine map: t->t_scale / t->t_shift must be NULL.
+ * transform_params [host] n_transform_params doubles; together with the likelihood's at most NNB_MAX_LIKE_PARAMS (else
+ * NNB_ERR_ARG).  NNB_ERR_STATE before nnb_set_user_transform.  Every kernel then runs the NVRTC-compiled variant.
+ */
+int nnb_set_target_user_transform(nnb_handle* h, int d, const nnb_target* t, const double* transform_params,
+                                  int n_transform_params);
+
+/*
+ * v = transform(u) of the target selected by nnb_set_target_user_transform (else NNB_ERR_STATE), formed exactly as the
+ * likelihood sees it, so the values equal the likelihood's x(i) bit for bit.
+ *   nnb_transform:       u [dev] n rows, float32 or float64 (in_f64), strides as nnb_loglike; out [dev] float64 (n, d)
+ *                        row-major.
+ *   nnb_transform_trace: trace_x [dev] float32 (T, d, n) as nnb_mcmc_run writes it; rows t_k = row0 + k * row_step,
+ *                        k < n_rows, into out [dev] float64 (n_rows, d, n) chain-minor.
+ * Stream-ordered and asynchronous.
+ */
+int nnb_transform(nnb_handle* h, const void* u, int in_f64, int64_t u_rs, int64_t u_cs, double* out, int64_t n,
+                  void* stream);
+int nnb_transform_trace(nnb_handle* h, const float* trace_x, int64_t n, int64_t row0, int64_t row_step, int64_t n_rows,
+                        double* out, void* stream);
+
+/*
  * logl[r] = safe_loglike(u[r]) for n rows (nnest/sampler.py:110-133): non-finite values become
  * -1e100 (-inf when the reference's result would be float32).  u [dev] n x d, float32 or float64
  * (in_f64); logl [dev] float64 n.  logp (may be NULL) [dev] float64 n receives safe_prior: 0 or -inf.

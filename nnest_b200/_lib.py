@@ -85,6 +85,13 @@ SYMBOLS = {
     'nnb_derived': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
     'nnb_derived_trace': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                     C.c_void_p, C.c_void_p]),
+    'nnb_set_user_transform': (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_int)]),
+    'nnb_user_transform_check': (C.c_int, [C.c_char_p, C.c_char_p, C.c_size_t]),
+    'nnb_set_target_user_transform': (C.c_int, [C.c_void_p, C.c_int, C.POINTER(nnb_target), C.c_void_p, C.c_int]),
+    'nnb_transform': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                C.c_void_p]),
+    'nnb_transform_trace': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                      C.c_void_p]),
     'nnb_loglike': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
                               C.c_int64, C.c_void_p]),
     'nnb_mcmc_init': (C.c_int, [C.c_void_p, C.POINTER(nnb_mcmc_init_args), C.c_void_p]),

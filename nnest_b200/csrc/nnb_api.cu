@@ -174,11 +174,20 @@ extern "C" int nnb_set_flow(nnb_handle* h, int d, int hidden, int num_layers, in
   return nnb_warp_pack(h, weights);
 }
 
-extern "C" int nnb_set_target(nnb_handle* h, int d, const nnb_target* t) {
+// user: the handle's user transform with its n_tp params tp replaces t_scale / t_shift (nnb_set_target_user_transform)
+static int set_target(nnb_handle* h, int d, const nnb_target* t, bool user, const double* tp, int n_tp) {
   if (!h || !t) return NNB_ERR_ARG;
   if (d < 1 || d > NNB_MAX_DIM) return fail(h, NNB_ERR_ARG, "x_dim must be in [1, NNB_MAX_DIM]");
-  if (t->like_id == NNB_LIKE_USER && !h->jit)
+  if (t->like_id == NNB_LIKE_USER && !nnb_jit_has_source(h, true))
     return fail(h, NNB_ERR_STATE, "NNB_LIKE_USER: no user likelihood installed (nnb_set_user_likelihood)");
+  if (user) {
+    if (!nnb_jit_has_source(h, false))
+      return fail(h, NNB_ERR_STATE, "no user transform installed (nnb_set_user_transform)");
+    if (t->t_scale || t->t_shift) return fail(h, NNB_ERR_ARG, "a user transform replaces t_scale / t_shift");
+    if (n_tp < 0 || (n_tp && !tp)) return fail(h, NNB_ERR_ARG, "bad transform parameter array");
+    if (t->n_like_params >= 0 && t->n_like_params + n_tp > NNB_MAX_LIKE_PARAMS)
+      return fail(h, NNB_ERR_ARG, "the likelihood's and the transform's parameters together exceed NNB_MAX_LIKE_PARAMS");
+  }
   if (t->n_like_params < 0 || t->n_like_params > NNB_MAX_LIKE_PARAMS || (t->n_like_params && !t->like_params))
     return fail(h, NNB_ERR_ARG, "bad likelihood parameter array");
   int need = 0;
@@ -208,8 +217,13 @@ extern "C" int nnb_set_target(nnb_handle* h, int d, const nnb_target* t) {
   TargetDesc td{};
   td.like_id = t->like_id; td.n_params = t->n_like_params; td.compute_f64 = t->compute_f64 ? 1 : 0;
   td.prior_kind = t->prior_kind; td.has_transform = t->t_scale ? 1 : 0; td.d = d;
+  if (user) {   // the transform's params follow the likelihood's; ts[0] says where they begin (TargetDesc)
+    td.has_transform = kTransformUser;
+    td.n_params += n_tp;
+  }
   std::vector<double> buf((size_t)target_doubles(d, td.n_params), 0.0);
-  for (int i = 0; i < td.n_params; ++i) buf[i] = t->like_params[i];
+  for (int i = 0; i < t->n_like_params; ++i) buf[i] = t->like_params[i];
+  for (int i = 0; user && i < n_tp; ++i) buf[t->n_like_params + i] = tp[i];
   double* ts = buf.data() + td.n_params;
   for (int i = 0; i < d; ++i) {
     ts[i] = t->t_scale ? t->t_scale[i] : 1.0;
@@ -217,6 +231,7 @@ extern "C" int nnb_set_target(nnb_handle* h, int d, const nnb_target* t) {
     ts[2 * d + i] = t->prior_lo ? t->prior_lo[i] : -INFINITY;
     ts[3 * d + i] = t->prior_hi ? t->prior_hi[i] : INFINITY;
   }
+  if (user) ts[0] = (double)t->n_like_params;
   {  // float32 mirrors behind the doubles (see TargetSmem)
     float* ff = reinterpret_cast<float*>(ts + 4 * d);
     for (int i = 0; i < d; ++i) {
@@ -235,6 +250,15 @@ extern "C" int nnb_set_target(nnb_handle* h, int d, const nnb_target* t) {
   h->tdesc = td;
   h->has_target = true;
   return NNB_OK;
+}
+
+extern "C" int nnb_set_target(nnb_handle* h, int d, const nnb_target* t) {
+  return set_target(h, d, t, false, nullptr, 0);
+}
+
+extern "C" int nnb_set_target_user_transform(nnb_handle* h, int d, const nnb_target* t, const double* transform_params,
+                                             int n_transform_params) {
+  return set_target(h, d, t, true, transform_params, n_transform_params);
 }
 
 template <bool INV>

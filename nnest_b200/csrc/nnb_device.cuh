@@ -66,6 +66,21 @@ __host__ __device__ inline int net_floats(int d, int H, int L, int k) {
 struct TargetDesc {
   int like_id, n_params, compute_f64, prior_kind, has_transform, d;
 };
+// has_transform: 0 none, 1 the affine map ts / tb, kTransformUser the handle's user transform (nnb_set_user_transform).
+// Only the run-time build (nnb_jit.cu, NNB_USER_TRANSFORM) evaluates a user transform; the launchers never hand such a
+// target to an ahead-of-time kernel (nnb_kernel, nnb_host.h).  Its params follow the likelihood's in `params`
+// (n_params counts both) and ts[0] holds the likelihood's count, i.e. where the transform's params begin.
+constexpr int kTransformUser = 2;
+
+// false when the target's transform is the user's: the fast paths that apply ts / tb themselves test it (always true in
+// the ahead-of-time build, which has no user transform)
+__device__ __forceinline__ bool builtin_transform(const TargetDesc& td) {
+#ifdef NNB_USER_TRANSFORM
+  return td.has_transform != kTransformUser;
+#else
+  return true;
+#endif
+}
 struct TargetSmem {
   TargetDesc desc;
   const double* params;  // [n_params]
@@ -317,12 +332,26 @@ template <> struct Ar<double> {
   static __device__ __forceinline__ double cosv(double a) { return cos(a); }
 };
 
-// v_i = transform(u)_i in T  (safe_transform, sampler.py:100-108; affine maps run.py:25-44, mcmc.py:111)
+#ifdef NNB_USER_TRANSFORM
+// u(j): coordinate j of the unit-box point in T, the argument nnb_user_transform reads
+template <typename T, typename XG>
+struct UnitRow {
+  const XG& xg;
+  __device__ __forceinline__ T operator()(int j) const { return (T)xg(j); }
+};
+#endif
+
+// v_i = transform(u)_i in T  (safe_transform, sampler.py:100-108; affine maps run.py:25-44, mcmc.py:111).  A user
+// transform (nnest_b200.likelihoods.CudaTransform) is evaluated afresh on every call: no per-chain buffer holds v.
 template <typename T, typename XG>
 struct Transformed {
   const TargetSmem& tg;
   const XG& xg;
   __device__ __forceinline__ T operator()(int i) const {
+#ifdef NNB_USER_TRANSFORM
+    if (tg.desc.has_transform == kTransformUser)
+      return nnb_user_transform(UnitRow<T, XG>{xg}, i, tg.desc.d, tg.params + (int)tg.ts[0]);
+#endif
     T u = (T)xg(i);
     if (!tg.desc.has_transform) return u;
     if (sizeof(T) == 4) return Ar<T>::add(Ar<T>::mul(u, (T)tg.tsf[i]), (T)tg.tbf[i]);

@@ -69,6 +69,8 @@ void nnb_jit_free(nnb_handle* h);                                               
 // the kernel `name` (a template instantiation, e.g. "mcmc_kernel<16, 0>") compiled around the handle's user likelihood;
 // nullptr with *rc set on failure
 const void* nnb_user_kernel(nnb_handle* h, const std::string& name, int* rc);          // nnb_jit.cu
+// whether the handle holds a user likelihood (like) / a user transform (!like) source                   nnb_jit.cu
+bool nnb_jit_has_source(const nnb_handle* h, bool like);
 int nnb_spline_flow(nnb_handle* h, bool inverse, const float* in, int64_t irs, int64_t ics, float* out, int64_t ors,
                     int64_t ocs, float* logdet, int* empty_out, int64_t n, cudaStream_t st);      // nnb_spline.cu
 int nnb_spline_init(nnb_handle* h, const InitParams& p, cudaStream_t st);              // nnb_spline.cu
@@ -99,12 +101,13 @@ static inline cudaError_t nnb_set_smem(K kernel, size_t bytes) {
   return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
-// The kernel a launcher runs: `builtin` (the ahead-of-time instantiation), or with the user likelihood selected
-// (NNB_LIKE_USER) the same instantiation compiled by NVRTC around the user's source.  `fmt`/`args` spell the
-// instantiation, e.g. ("mcmc_kernel<%d, %d>", H, MODE).  nullptr with *rc set on failure.
+// The kernel a launcher runs: `builtin` (the ahead-of-time instantiation), or with the user likelihood (NNB_LIKE_USER)
+// or the user transform (nnb_set_target_user_transform) selected the same instantiation compiled by NVRTC around the
+// user's sources.  `fmt`/`args` spell the instantiation, e.g. ("mcmc_kernel<%d, %d>", H, MODE).  nullptr with *rc set on
+// failure.
 template <typename... A>
 static inline const void* nnb_kernel(nnb_handle* h, const void* builtin, int* rc, const char* fmt, A... args) {
-  if (h->tdesc.like_id != NNB_LIKE_USER) return builtin;
+  if (h->tdesc.like_id != NNB_LIKE_USER && h->tdesc.has_transform != nnb::kTransformUser) return builtin;
   char name[128];
   snprintf(name, sizeof(name), fmt, args...);
   return nnb_user_kernel(h, name, rc);

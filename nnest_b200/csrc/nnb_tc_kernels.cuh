@@ -788,7 +788,8 @@ mcmc_tc_kernel(TcFlowDesc f, const float* __restrict__ wglob, TargetDesc td, con
           if (ratio > 1.0f) ratio = 1.0f;
           const bool m1 = u01 < ratio;
           if (m1) {
-            if (DD > 0 && td.like_id == NNB_LIKE_ROSENBROCK && !td.compute_f64 && td.has_transform) {
+            if (DD > 0 && td.like_id == NNB_LIKE_ROSENBROCK && !td.compute_f64 && td.has_transform &&
+                builtin_transform(td)) {
               // the config-4 target inline (same arithmetic as loglike_T<float>: likelihoods.py:50-51 after the float32
               // affine transform), transform coefficients as constant-bank operands
               // The terms i = 1 .. N run as packed FP32 pairs (i, i + h), h = ceil(N / 2): with V_m = (x_m, x_{m+h}) a pair's

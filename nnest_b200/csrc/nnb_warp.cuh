@@ -199,7 +199,7 @@ mcmc_warp_kernel(WarpFlowDesc f, const float* __restrict__ wglob, TargetDesc td,
     }
   };
   draw(p.step_offset + (unsigned int)(p.s0 + 1), p.s0);
-  const bool fast_rosen = tg.desc.like_id == NNB_LIKE_ROSENBROCK && !tg.desc.compute_f64;
+  const bool fast_rosen = tg.desc.like_id == NNB_LIKE_ROSENBROCK && !tg.desc.compute_f64 && builtin_transform(tg.desc);
 
   for (int s = p.s0 + 1; s <= p.s0 + p.nsteps; ++s) {
     const unsigned int step_abs = p.step_offset + (unsigned int)s;

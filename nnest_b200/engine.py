@@ -294,13 +294,27 @@ class Engine(object):
         self.num_derived = int(num_derived)
         return n.value
 
+    def set_user_transform(self, source):
+        """Install a CUDA C++ prior transform (nnb_set_user_transform): returns the number of kernel variants compiled."""
+        n = C.c_int(0)
+        self._check(self.lib.nnb_set_user_transform(self.h, source.encode(), C.byref(n)))
+        self.transform_source = source
+        return n.value
+
     def set_target(self, d, like_id, like_params=(), t_scale=None, t_shift=None, compute_f64=False,
-                   prior_kind=L.NNB_PRIOR_NONE, prior_lo=None, prior_hi=None, user_source=None, num_derived=0):
+                   prior_kind=L.NNB_PRIOR_NONE, prior_lo=None, prior_hi=None, user_source=None, num_derived=0,
+                   transform_source=None, transform_params=()):
         """user_source: CUDA C++ of the likelihood NNB_LIKE_USER selects (with num_derived derived parameters), installed
-        first when it is not the current one."""
+        first when it is not the current one.  transform_source: CUDA C++ of a prior transform, used with its
+        transform_params in place of t_scale / t_shift (nnb_set_target_user_transform), installed first likewise."""
         if user_source is not None and (user_source, num_derived) != (getattr(self, 'user_source', None),
                                                                        getattr(self, 'num_derived', 0)):
             self.set_user_likelihood(user_source, num_derived)
+        if transform_source is not None:
+            if t_scale is not None or t_shift is not None:
+                raise ValueError('a user transform replaces t_scale / t_shift')
+            if transform_source != getattr(self, 'transform_source', None):
+                self.set_user_transform(transform_source)
         t = L.nnb_target()
         keep = []
         t.like_id = like_id
@@ -320,8 +334,46 @@ class Engine(object):
             keep.append(a)
             a, t.prior_hi = _darr(np.broadcast_to(prior_hi, (d,)))
             keep.append(a)
-        self._check(self.lib.nnb_set_target(self.h, d, C.byref(t)))
+        if transform_source is not None:
+            a, tp = _darr(transform_params if len(transform_params) else [0.0])
+            keep.append(a)
+            self._check(self.lib.nnb_set_target_user_transform(self.h, d, C.byref(t), tp, len(transform_params)))
+        else:
+            self._check(self.lib.nnb_set_target(self.h, d, C.byref(t)))
         self.target_d = d
+
+    def transform(self, u, out=None):
+        """u (n,d) float32 or float64 cuda -> v = transform(u) float64 (n, d) of the target's user transform
+        (nnb_transform): the values the likelihood sees at these points, bit for bit."""
+        assert u.is_cuda and u.dim() == 2 and u.shape[1] == self.target_d
+        assert u.dtype in (torch.float32, torch.float64)
+        n, d = u.shape
+        if out is None:
+            out = torch.empty((n, d), dtype=torch.float64, device=u.device)
+        assert out.dtype == torch.float64 and out.is_contiguous() and tuple(out.shape) == (n, d)
+        if n:
+            self._check(self.lib.nnb_transform(self.h, _ptr(u), 1 if u.dtype == torch.float64 else 0, u.stride(0),
+                                               u.stride(1), _ptr(out), n, _stream()))
+            self.gpu_launches += 1
+        return out
+
+    def transform_trace(self, trace_x, row0=0, row_step=1, n_rows=None, out=None):
+        """v = transform(x) of rows row0, row0 + row_step, ... (n_rows of them; default: to the end) of a device trace
+        float32 (T, d, n) -> float64 (n_rows, d, n) (nnb_transform_trace)."""
+        assert trace_x.is_cuda and trace_x.dtype == torch.float32 and trace_x.is_contiguous() and trace_x.dim() == 3
+        T, d, n = trace_x.shape
+        assert d == self.target_d
+        if n_rows is None:
+            n_rows = len(range(row0, T, row_step))
+        assert n_rows == 0 or row0 + (n_rows - 1) * row_step < T
+        if out is None:
+            out = torch.empty((n_rows, d, n), dtype=torch.float64, device=trace_x.device)
+        assert out.dtype == torch.float64 and out.is_contiguous() and tuple(out.shape) == (n_rows, d, n)
+        if n and n_rows:
+            self._check(self.lib.nnb_transform_trace(self.h, _ptr(trace_x), n, row0, row_step, n_rows, _ptr(out),
+                                                     _stream()))
+            self.gpu_launches += 1
+        return out
 
     def loglike(self, u, want_prior=False):
         """u (n,d) float32 or float64 cuda -> logl float64 (n,) [, logp float64 (n,)]"""

@@ -252,3 +252,76 @@ class CudaLikelihood(Likelihood):
         if self._max_loglike is None:
             raise AttributeError('max_loglike was not given to CudaLikelihood')
         return self._max_loglike
+
+
+class CudaTransform(object):
+    """A prior transform written in CUDA C++ -- the sampler's `transform`, from the unit box [-1, 1]^x_dim to the physical
+    parameters -- compiled at run time (NVRTC) into the library's own kernels, next to the likelihood.
+
+    `source` defines
+
+        template <typename U>
+        __device__ auto nnb_user_transform(const U& u, int i, int d, const double* params) -> decltype(u(0));
+
+    which returns coordinate i of v = transform(u).  u(j) is coordinate j of the unit-box point, a float or a double
+    (`decltype(u(0))` names it); any u(j) may be read, so transforms that mix coordinates (a Cholesky factor) are allowed.
+    Nothing stores v: every x(i) a likelihood (built-in or CudaLikelihood), the prior or nnb_user_derived reads evaluates
+    the transform once, so x(i) costs one transform evaluation per call -- a likelihood that reads a coordinate several
+    times does well to keep it in a local variable.  `params` (at most NNB_MAX_LIKE_PARAMS doubles, and together with
+    the likelihood's at most that many) reach the function as `params`; larger constants belong in the source as
+    __constant__ arrays.  Write float arithmetic with the *_rn intrinsics where the exact rounding matters.
+
+    float64=True (the default): float32 points are promoted to double before the transform, so the transform, the
+    likelihood, the prior and the derived parameters all compute in double.  float64=False: the arithmetic follows the
+    input, float for float32 points, as the float32 affine maps do.
+
+    Calling the object maps host rows (n, x_dim) or (x_dim,) on the device: float64 out when float64=True or the input is
+    float64, float32 otherwise (NumPy's dtype rules for the callable it replaces).  In a sampler the values are those the
+    likelihood saw, bit for bit.  The source is compiled once here, without a device: a source that does not compile
+    raises ValueError with the compiler's log.  Compiled kernels are cached as for CudaLikelihood.
+    """
+
+    def __init__(self, x_dim, source, params=(), float64=True):
+        import ctypes as C
+        params = [float(p) for p in np.asarray(params, dtype=np.float64).ravel()]
+        if len(params) > L.NNB_MAX_LIKE_PARAMS:
+            raise ValueError('CudaTransform takes at most %d params, got %d' % (L.NNB_MAX_LIKE_PARAMS, len(params)))
+        if not isinstance(source, str) or not source.strip():
+            raise ValueError('source must be a non-empty string of CUDA C++')
+        log = C.create_string_buffer(1 << 16)
+        rc = L.load().nnb_user_transform_check(source.encode(), log, len(log))
+        if rc == L.NNB_ERR_UNSUPPORTED:
+            raise RuntimeError('CudaTransform needs NVRTC (libnvrtc.so.12), which could not be loaded')
+        if rc != L.NNB_OK:
+            raise ValueError('the transform source does not compile:\n' + log.value.decode(errors='replace'))
+        self.x_dim = int(x_dim)
+        self.source = source
+        self.params = params
+        self.float64 = bool(float64)
+
+    def install(self, engine, d, like_id, like_params=(), **target):
+        """Select this transform on `engine`'s target (Engine.set_target with it in place of t_scale / t_shift)."""
+        engine.set_target(d, like_id, like_params, compute_f64=self.float64, transform_source=self.source,
+                          transform_params=self.params, **target)
+
+    def apply(self, engine, u):
+        """Host rows through `engine`, whose target already holds this transform -> host rows (see the class docs)."""
+        import torch
+        if isinstance(u, list):
+            u = np.array(u)
+        u = np.asarray(u)
+        single = u.ndim == 1
+        uu = np.ascontiguousarray(u[None, :] if single else u)
+        if uu.dtype not in (np.float32, np.float64):
+            uu = uu.astype(np.float64)
+        if uu.ndim != 2 or uu.shape[1] != self.x_dim:
+            raise ValueError('CudaTransform maps (n, %d) rows, got shape %s' % (self.x_dim, u.shape))
+        v = engine.transform(torch.from_numpy(uu).to(engine.device)).cpu().numpy()
+        if not self.float64 and uu.dtype == np.float32:
+            v = v.astype(np.float32)
+        return v[0] if single else v
+
+    def __call__(self, u):
+        eng = _eval_engine()
+        self.install(eng, self.x_dim, L.NNB_LIKE_ROSENBROCK)
+        return self.apply(eng, u)

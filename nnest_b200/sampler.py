@@ -9,7 +9,8 @@ What is kept from the reference's contract (SURVEY.md section 8b):
 What differs, by design (north_star: no CPU fallback):
   * `loglike` must be one of nnest_b200.likelihoods (the batched CUDA likelihood library) and `transform`
     must be a per-dimension affine map (probed numerically: the maps of examples/nested/run.py:25-44 and
-    nnest/mcmc.py:111 all are); anything else raises NotImplementedError;
+    nnest/mcmc.py:111 all are) or a CudaTransform, a prior transform written in CUDA C++ (Gaussian, log-uniform,
+    correlated priors ...); anything else raises NotImplementedError;
   * random numbers come from a per-chain Philox stream (seed = `seed` kwarg), not torch's global generator.
 """
 from __future__ import division, print_function
@@ -23,7 +24,7 @@ import torch
 
 from . import _lib as L
 from . import dist
-from .likelihoods import CudaLikelihood, Likelihood
+from .likelihoods import CudaLikelihood, CudaTransform, Likelihood
 from .priors import UniformPrior
 from .trainer import Trainer
 from .utils.evaluation import acceptance_rate, effective_sample_size, mean_jump_distance
@@ -50,7 +51,8 @@ def probe_affine_transform(transform, d):
     tol = 1e-9 * (1.0 + np.abs(want).max())
     if want.shape != pts.shape or np.abs(want - got).max() > tol:
         raise NotImplementedError('transform is not a per-dimension affine map; arbitrary Python transforms '
-                                  'cannot run inside the CUDA step kernel (no CPU fallback)')
+                                  'cannot run inside the CUDA step kernel (no CPU fallback): write it in CUDA C++ as a '
+                                  'nnest_b200.likelihoods.CudaTransform')
     return scale, shift, promotes
 
 
@@ -181,8 +183,26 @@ class Sampler(object):
     @transform.setter
     def transform(self, fn):
         """Assigning `sampler.transform = ...` (as MCMCSampler.run does, nnest/mcmc.py:111) re-probes the map and
-        re-installs likelihood + transform + prior on the device."""
+        re-installs likelihood + transform + prior on the device.  A CudaTransform is installed as it is (not probed);
+        `sampler.transform(u)` then evaluates it through the sampler's own engine, so the values are those the
+        likelihood saw."""
         self._user_transform = fn
+        self._cuda_transform = fn if isinstance(fn, CudaTransform) else None
+        if self._cuda_transform is not None:
+            if fn.x_dim != self.x_dim:
+                raise ValueError('the CudaTransform has x_dim %d, the sampler %d' % (fn.x_dim, self.x_dim))
+            self._t_scale, self._t_shift, self._t_f64 = None, None, fn.float64
+
+            def cuda_transform(x):
+                if isinstance(x, list):
+                    x = np.array(x)
+                if len(x.shape) == 1:
+                    assert x.shape[0] == self.x_dim
+                    x = np.expand_dims(x, 0)
+                return fn.apply(self.engine, x)
+            self._transform_fn = cuda_transform
+            self._install_target()
+            return
         scale, shift, promotes = probe_affine_transform(fn, self.x_dim)
         self._t_scale, self._t_shift, self._t_f64 = scale, shift, promotes
 
@@ -214,6 +234,11 @@ class Sampler(object):
             kind = L.NNB_PRIOR_BOX_V if (self._transform_prior and self._user_transform is not None) \
                 else L.NNB_PRIOR_BOX_U
             lo, hi = prior.minimum.astype(np.float64), prior.maximum.astype(np.float64)
+        if self._cuda_transform is not None:
+            self._cuda_transform.install(self.engine, self.x_dim, self._like.like_id, self._like.device_params(),
+                                         prior_kind=kind, prior_lo=lo, prior_hi=hi,
+                                         user_source=self._like.device_source(), num_derived=self.num_derived)
+            return
         self.engine.set_target(self.x_dim, self._like.like_id, self._like.device_params(), t_scale=self._t_scale,
                                t_shift=self._t_shift, compute_f64=self._t_f64, prior_kind=kind, prior_lo=lo,
                                prior_hi=hi, user_source=self._like.device_source(), num_derived=self.num_derived)
@@ -390,7 +415,13 @@ class Sampler(object):
                 self._save_samples(self.transform(full.reshape(-1, self.x_dim)).reshape(st.n, it + 1, self.x_dim),
                                    out['trace_logl'][:it + 1].cpu().numpy().transpose(1, 0), derived_samples=der)
             if stats_interval is not None and it % stats_interval == 0:
-                self._chain_stats(None, step=it, trace=self._device_trace, t_scale=ts, t_shift=tb)
+                if self._cuda_transform is not None:
+                    # statistics of the transformed samples (the reference's): the transform on the device, the
+                    # statistics on the host (utils/evaluation.py) -- a diagnostic, not the hot path
+                    v = self.engine.transform_trace(self._device_trace, 0, 1, it + 1).cpu().numpy()
+                    self._chain_stats(v.transpose(2, 0, 1), step=it)
+                else:
+                    self._chain_stats(None, step=it, trace=self._device_trace, t_scale=ts, t_shift=tb)
         return samples, latent_samples, derived_samples, loglikes, out['scale'], ncall
 
     _STAGE_BYTES = 128 << 20
