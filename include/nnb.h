@@ -159,7 +159,9 @@ int nnb_set_target(nnb_handle* h, int d, const nnb_target* t);
  *     template <typename X> __device__ double nnb_user_loglike(const X& x, int d, const double* params);
  * x(i) is coordinate i after the target's transform, in the arithmetic type the built-in likelihoods see at the same place
  * (float when compute_f64 == 0 and the input is float32, double otherwise); params are the target's like_params (up to
- * NNB_MAX_LIKE_PARAMS).  Larger constants go into the source as __constant__ arrays.  A non-finite result becomes -inf
+ * NNB_MAX_LIKE_PARAMS).  Data of any size -- observations, a covariance -- goes into device arrays the source reads as
+ * nnb_data.<name>[j] (nnb_set_user_likelihood_data below); a small table of fixed constants may also be written into the
+ * source as a __constant__ array (64 KB per module, and a new table is a new source to compile).  A non-finite result becomes -inf
  * when x(i) is float and -1e100 otherwise, as for the built-in likelihoods.
  * nnb_set_user_likelihood installs the source on the handle; nnb_set_target with like_id NNB_LIKE_USER then selects it
  * (NNB_ERR_STATE before a source is installed).  NVRTC compiles the library's own kernel templates around the source:
@@ -190,6 +192,40 @@ int nnb_user_likelihood_check(const char* source, char* log, size_t cap);
  */
 int nnb_set_user_likelihood_derived(nnb_handle* h, const char* source, int num_derived, int* n_compiled_out);
 int nnb_user_likelihood_check_derived(const char* source, int num_derived, char* log, size_t cap);
+
+/*
+ * A dataset of a user likelihood: up to NNB_MAX_DATA_ARRAYS named, typed, read-only device arrays.  With n_arrays > 0
+ * the source is compiled behind generated declarations (the file user_data.cuh):
+ *     template <typename T> struct nnb_span {        // T: double, float or int (NNB_DTYPE_F64 / _F32 / _I32)
+ *       const T* p; long long n;
+ *       __device__ T operator[](long long j) const;  // p[j] through the read-only data path
+ *       __device__ long long size() const;           // n
+ *     };
+ *     struct nnb_user_data_t { nnb_span<T0> <name0>; nnb_span<T1> <name1>; ... };   // in the order given
+ *     __constant__ nnb_user_data_t nnb_data;
+ * so nnb_user_loglike and nnb_user_derived read array k as nnb_data.<name k>[j] and its length as .size().  A user
+ * transform does not see nnb_data.  names [host] are C identifiers, none repeated; dtypes [host] NNB_DTYPE_*.  The layout
+ * (names and dtypes) is compiled in, and the cache keys name it; the values, sizes and pointers are not, so a new
+ * dataset of the same layout needs no compile.
+ * nnb_set_user_likelihood_data is nnb_set_user_likelihood_derived with that layout; n_arrays == 0 is exactly
+ * nnb_set_user_likelihood_derived.  A bad layout (a name that is not an identifier or repeats, an unknown dtype, more
+ * than NNB_MAX_DATA_ARRAYS arrays) is NNB_ERR_ARG.  Installing a source or layout drops the dataset's binding.
+ * nnb_user_likelihood_check_data checks the same without a handle or a device, as nnb_user_likelihood_check does: a
+ * source that reads an undeclared array, or an array as the wrong type, is refused with NVRTC's log.
+ * nnb_bind_user_data binds the dataset: ptrs [host] n_arrays pointers to device (or managed) memory of the handle's
+ * device, each aligned to its element size (NULL only for an empty array); sizes [host] n_arrays element counts >= 0.
+ * Anything else is NNB_ERR_ARG, checked on the host.  The table is written into every loaded kernel module that holds
+ * the likelihood, and into later ones as they load.  Synchronous, and ordered as nnb_set_target.  The caller owns the
+ * arrays and keeps them alive and unchanged while launches that read them are in flight.  A launch that needs the
+ * likelihood of a layout with arrays before nnb_bind_user_data is NNB_ERR_STATE, refused before anything runs.
+ */
+#define NNB_MAX_DATA_ARRAYS 16
+enum { NNB_DTYPE_F64 = 0, NNB_DTYPE_F32 = 1, NNB_DTYPE_I32 = 2 };
+int nnb_set_user_likelihood_data(nnb_handle* h, const char* source, int num_derived, int n_arrays,
+                                 const char* const* names, const int* dtypes, int* n_compiled_out);
+int nnb_user_likelihood_check_data(const char* source, int num_derived, int n_arrays, const char* const* names,
+                                   const int* dtypes, char* log, size_t cap);
+int nnb_bind_user_data(nnb_handle* h, const void* const* ptrs, const int64_t* sizes);
 
 /*
  * derived values of the target selected by nnb_set_target (like_id NNB_LIKE_USER with num_derived > 0, else

@@ -14,6 +14,8 @@ NNB_MAX_DIM = 128
 NNB_MAX_BLOCKS = 16
 NNB_MAX_LIKE_PARAMS = 160
 NNB_MAX_DERIVED = 32
+NNB_MAX_DATA_ARRAYS = 16
+NNB_DTYPE_F64, NNB_DTYPE_F32, NNB_DTYPE_I32 = 0, 1, 2
 
 NNB_OK, NNB_ERR_ARG, NNB_ERR_CUDA, NNB_ERR_STATE, NNB_ERR_UNSUPPORTED, NNB_ERR_START = 0, -1, -2, -3, -4, -5
 NNB_FLOW_TRANSLATE_ONLY, NNB_FLOW_CONST_SCALE = 1, 2
@@ -82,6 +84,11 @@ SYMBOLS = {
     'nnb_user_likelihood_check': (C.c_int, [C.c_char_p, C.c_char_p, C.c_size_t]),
     'nnb_set_user_likelihood_derived': (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.POINTER(C.c_int)]),
     'nnb_user_likelihood_check_derived': (C.c_int, [C.c_char_p, C.c_int, C.c_char_p, C.c_size_t]),
+    'nnb_set_user_likelihood_data': (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.POINTER(C.c_char_p),
+                                               C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    'nnb_user_likelihood_check_data': (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_int),
+                                                 C.c_char_p, C.c_size_t]),
+    'nnb_bind_user_data': (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), _ip]),
     'nnb_derived': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
     'nnb_derived_trace': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                     C.c_void_p, C.c_void_p]),

@@ -98,6 +98,8 @@ class Engine(object):
         self.h = h
         self.d = None
         self.num_derived = 0      # derived parameters of the installed user likelihood
+        self.user_layout = ()     # (name, NNB_DTYPE_*) of its dataset's arrays
+        self._data_token, self._data_tensors = None, ()   # the bound dataset (UserData.token) and its device copy
         self.gpu_launches = 0     # kernels launched through this engine (bench.py reports it)
         self.default_impl = int(os.environ.get('NNB_IMPL', L.NNB_IMPL_AUTO))   # 0 auto, 1 ffma, 2 tcgen05
 
@@ -282,17 +284,41 @@ class Engine(object):
         return acceptance, T / ess, jump_distance
 
     # ---- target -----------------------------------------------------------------------------
-    def set_user_likelihood(self, source, num_derived=0):
-        """Install a CUDA C++ likelihood (nnb_set_user_likelihood, or nnb_set_user_likelihood_derived with num_derived > 0):
-        returns the number of kernel variants compiled."""
+    def set_user_likelihood(self, source, num_derived=0, layout=()):
+        """Install a CUDA C++ likelihood (nnb_set_user_likelihood, or nnb_set_user_likelihood_derived with num_derived > 0,
+        or nnb_set_user_likelihood_data with a dataset layout: (name, NNB_DTYPE_*) per array): returns the number of
+        kernel variants compiled.  Drops the bound dataset."""
         n = C.c_int(0)
-        if num_derived:
+        layout = tuple(layout)
+        self.user_source = None     # until the call succeeds: the library keeps the previous source on failure, unbound
+        self._data_token, self._data_tensors = None, ()
+        if layout:
+            names = (C.c_char_p * len(layout))(*[name.encode() for name, _ in layout])
+            dtypes = (C.c_int * len(layout))(*[dt for _, dt in layout])
+            self._check(self.lib.nnb_set_user_likelihood_data(self.h, source.encode(), int(num_derived), len(layout),
+                                                               names, dtypes, C.byref(n)))
+        elif num_derived:
             self._check(self.lib.nnb_set_user_likelihood_derived(self.h, source.encode(), int(num_derived), C.byref(n)))
         else:
             self._check(self.lib.nnb_set_user_likelihood(self.h, source.encode(), C.byref(n)))
         self.user_source = source
         self.num_derived = int(num_derived)
+        self.user_layout = layout
         return n.value
+
+    def bind_user_data(self, user_data):
+        """Upload a CudaLikelihood's dataset (likelihoods.UserData) to this engine's device and bind it
+        (nnb_bind_user_data).  The tensors stay alive until another dataset is bound; binding the dataset already bound
+        does nothing, so a dataset is uploaded once per engine however often the target is set."""
+        if user_data.token == self._data_token:
+            return
+        tensors = [torch.from_numpy(np.array(a)).to(self.device) for a in user_data.arrays]
+        n = len(tensors)
+        ptrs = (C.c_void_p * n)(*[t.data_ptr() if t.numel() else None for t in tensors])
+        sizes = (C.c_int64 * n)(*[t.numel() for t in tensors])
+        self._data_token = None
+        self._check(self.lib.nnb_bind_user_data(self.h, ptrs, sizes))
+        self._data_token, self._data_tensors = user_data.token, tuple(tensors)
 
     def set_user_transform(self, source):
         """Install a CUDA C++ prior transform (nnb_set_user_transform): returns the number of kernel variants compiled."""
@@ -303,13 +329,18 @@ class Engine(object):
 
     def set_target(self, d, like_id, like_params=(), t_scale=None, t_shift=None, compute_f64=False,
                    prior_kind=L.NNB_PRIOR_NONE, prior_lo=None, prior_hi=None, user_source=None, num_derived=0,
-                   transform_source=None, transform_params=()):
-        """user_source: CUDA C++ of the likelihood NNB_LIKE_USER selects (with num_derived derived parameters), installed
-        first when it is not the current one.  transform_source: CUDA C++ of a prior transform, used with its
+                   transform_source=None, transform_params=(), user_data=None):
+        """user_source: CUDA C++ of the likelihood NNB_LIKE_USER selects (with num_derived derived parameters and the
+        layout of user_data, a likelihoods.UserData), installed first when it is not the current one; user_data is then
+        uploaded and bound unless it already is.  transform_source: CUDA C++ of a prior transform, used with its
         transform_params in place of t_scale / t_shift (nnb_set_target_user_transform), installed first likewise."""
-        if user_source is not None and (user_source, num_derived) != (getattr(self, 'user_source', None),
-                                                                       getattr(self, 'num_derived', 0)):
-            self.set_user_likelihood(user_source, num_derived)
+        layout = user_data.layout if user_data is not None else ()
+        if user_source is not None and (user_source, num_derived, layout) != (getattr(self, 'user_source', None),
+                                                                               getattr(self, 'num_derived', 0),
+                                                                               getattr(self, 'user_layout', ())):
+            self.set_user_likelihood(user_source, num_derived, layout)
+        if user_source is not None and user_data is not None:
+            self.bind_user_data(user_data)
         if transform_source is not None:
             if t_scale is not None or t_shift is not None:
                 raise ValueError('a user transform replaces t_scale / t_shift')

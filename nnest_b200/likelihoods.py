@@ -4,11 +4,18 @@ per-row Python loop.  Each class only carries the id and parameter vector the ke
 instance on host arrays uploads them, runs the kernel and downloads the values -- there is no CPU
 implementation in this package.
 """
+import itertools
+import re
+
 import numpy as np
 
 from . import _lib as L
 
 _engines = {}
+_data_tokens = itertools.count(1)
+# the element types a dataset array may have, and their codes in the C ABI
+DATA_DTYPES = {np.dtype(np.float64): L.NNB_DTYPE_F64, np.dtype(np.float32): L.NNB_DTYPE_F32,
+               np.dtype(np.int32): L.NNB_DTYPE_I32}
 
 
 def _eval_engine():
@@ -38,6 +45,10 @@ class Likelihood(object):
         """CUDA C++ of a user likelihood (CudaLikelihood), None for the built-in ones."""
         return None
 
+    def device_data(self):
+        """The dataset of a CudaLikelihood (a UserData), None for the built-in likelihoods and without data."""
+        return None
+
     def __call__(self, x):
         """x: (n, x_dim) or (x_dim,) array in the likelihood's own coordinates -> log-likelihood(s)."""
         import torch
@@ -51,7 +62,7 @@ class Likelihood(object):
         self.num_evaluations += xx.shape[0]
         eng = _eval_engine()
         eng.set_target(self.x_dim, self.like_id, self.device_params(), user_source=self.device_source(),
-                       num_derived=self.num_derived)
+                       num_derived=self.num_derived, user_data=self.device_data())
         xd = torch.from_numpy(xx).to(eng.device)
         out = eng.loglike(xd).cpu().numpy()
         if self.follows_input_dtype and xx.dtype == np.float32:
@@ -199,9 +210,19 @@ class CudaLikelihood(Likelihood):
 
     where x(i) is coordinate i of the point after the sampler's affine transform -- a float when the target computes in
     float32 (float32 points, float32 transform), a double otherwise: `decltype(x(0))` names it -- and `params` holds the
-    `params` given here (at most NNB_MAX_LIKE_PARAMS doubles).  Larger constants, such as an inverse covariance, belong in
-    the source as __constant__ arrays.  A non-finite value is clamped as for the built-in likelihoods: to -inf when x(i)
-    is a float, to -1e100 otherwise.
+    `params` given here (at most NNB_MAX_LIKE_PARAMS doubles).  A non-finite value is clamped as for the built-in
+    likelihoods: to -inf when x(i) is a float, to -1e100 otherwise.
+
+    Data -- observations, an inverse covariance, anything larger than `params` -- goes into `data`: an ordered mapping
+    from name to array (at most NNB_MAX_DATA_ARRAYS of them).  The source reads array `name` as `nnb_data.name[j]` and
+    its length as `nnb_data.name.size()`, from nnb_user_loglike and nnb_user_derived alike.  Names are C identifiers;
+    each array keeps its dtype, which must be float64 (read as double), float32 (float) or int32 (int) -- convert other
+    types on purpose, e.g. an int64 index array with .astype(np.int32).  Arrays are flattened in C order and copied
+    here, so later changes to the caller's arrays change nothing; `data` holds the frozen copies.  Only the names and
+    dtypes are compiled in: another CudaLikelihood with the same source and the same names and dtypes, but other values
+    and sizes, reuses every compiled kernel, and switching between them costs one upload of the data to each device.
+    A __constant__ array in the source still works for a small table of fixed constants, but constant memory holds
+    64 KB, and a table written into the source makes every new table a new source to compile.
 
     num_derived > 0 (at most NNB_MAX_DERIVED): the source also defines
 
@@ -220,7 +241,7 @@ class CudaLikelihood(Likelihood):
     """
     like_id = L.NNB_LIKE_USER
 
-    def __init__(self, x_dim, source, params=(), max_loglike=None, num_derived=0):
+    def __init__(self, x_dim, source, params=(), data=None, max_loglike=None, num_derived=0):
         import ctypes as C
         params = [float(p) for p in np.asarray(params, dtype=np.float64).ravel()]
         if len(params) > L.NNB_MAX_LIKE_PARAMS:
@@ -229,8 +250,14 @@ class CudaLikelihood(Likelihood):
             raise ValueError('source must be a string of CUDA C++')
         if int(num_derived) != num_derived or not 0 <= num_derived <= L.NNB_MAX_DERIVED:
             raise ValueError('num_derived must be an integer in [0, %d], got %r' % (L.NNB_MAX_DERIVED, num_derived))
+        self._data = UserData(data) if data is not None and len(data) else None
         log = C.create_string_buffer(1 << 16)
-        rc = L.load().nnb_user_likelihood_check_derived(source.encode(), int(num_derived), log, len(log))
+        if self._data is None:
+            rc = L.load().nnb_user_likelihood_check_derived(source.encode(), int(num_derived), log, len(log))
+        else:
+            names, dtypes = self._data.c_layout()
+            rc = L.load().nnb_user_likelihood_check_data(source.encode(), int(num_derived), len(self._data.names),
+                                                         names, dtypes, log, len(log))
         if rc == L.NNB_ERR_UNSUPPORTED:
             raise RuntimeError('CudaLikelihood needs NVRTC (libnvrtc.so.12), which could not be loaded')
         if rc != L.NNB_OK:
@@ -247,11 +274,56 @@ class CudaLikelihood(Likelihood):
     def device_source(self):
         return self.source
 
+    def device_data(self):
+        return self._data
+
+    @property
+    def data(self):
+        """name -> the frozen flat copy of each dataset array ({} without data)"""
+        return dict(zip(self._data.names, self._data.arrays)) if self._data is not None else {}
+
     @property
     def max_loglike(self):
         if self._max_loglike is None:
             raise AttributeError('max_loglike was not given to CudaLikelihood')
         return self._max_loglike
+
+
+class UserData(object):
+    """The dataset of a CudaLikelihood, frozen at construction: names, NNB_DTYPE_* codes and read-only flat copies of the
+    arrays, with a token no other UserData has, so an engine uploads a given dataset at most once."""
+
+    def __init__(self, data):
+        items = list(data.items()) if hasattr(data, 'items') else list(data)
+        if len(items) > L.NNB_MAX_DATA_ARRAYS:
+            raise ValueError('CudaLikelihood takes at most %d data arrays, got %d' % (L.NNB_MAX_DATA_ARRAYS, len(items)))
+        names, arrays = [], []
+        for name, a in items:
+            if not isinstance(name, str) or not re.match(r'^[A-Za-z_][A-Za-z0-9_]*\Z', name):
+                raise ValueError('data array names must be C identifiers, got %r' % (name,))
+            if name in names:
+                raise ValueError('data array name %r is repeated' % name)
+            a = np.asarray(a)
+            if a.dtype not in DATA_DTYPES:
+                raise ValueError('data array %r has dtype %s; the accepted dtypes are float64, float32 and int32 (convert '
+                                 'others on purpose, e.g. .astype(np.int32))' % (name, a.dtype))
+            a = np.array(a, order='C', copy=True).ravel()
+            a.flags.writeable = False
+            names.append(name)
+            arrays.append(a)
+        self.names, self.arrays = tuple(names), tuple(arrays)
+        self.dtypes = tuple(DATA_DTYPES[a.dtype] for a in arrays)
+        self.token = next(_data_tokens)
+
+    @property
+    def layout(self):
+        """(name, NNB_DTYPE_*) per array: what the compiled kernels depend on"""
+        return tuple(zip(self.names, self.dtypes))
+
+    def c_layout(self):
+        import ctypes as C
+        n = len(self.names)
+        return (C.c_char_p * n)(*[s.encode() for s in self.names]), (C.c_int * n)(*self.dtypes)
 
 
 class CudaTransform(object):

@@ -237,11 +237,13 @@ class Sampler(object):
         if self._cuda_transform is not None:
             self._cuda_transform.install(self.engine, self.x_dim, self._like.like_id, self._like.device_params(),
                                          prior_kind=kind, prior_lo=lo, prior_hi=hi,
-                                         user_source=self._like.device_source(), num_derived=self.num_derived)
+                                         user_source=self._like.device_source(), num_derived=self.num_derived,
+                                         user_data=self._like.device_data())
             return
         self.engine.set_target(self.x_dim, self._like.like_id, self._like.device_params(), t_scale=self._t_scale,
                                t_shift=self._t_shift, compute_f64=self._t_f64, prior_kind=kind, prior_lo=lo,
-                               prior_hi=hi, user_source=self._like.device_source(), num_derived=self.num_derived)
+                               prior_hi=hi, user_source=self._like.device_source(), num_derived=self.num_derived,
+                               user_data=self._like.device_data())
 
     def _to_device_rows(self, x):
         if isinstance(x, list):
